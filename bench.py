@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- LM iterations/s of the bundle-adjustment hot path on B200 (and the CPU reference arm beside it).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg5] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg5] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W     (one rank per GPU)
 
 A "step" is ONE Levenberg-Marquardt iteration (one row of Ceres' progress table: Schur elimination of the
@@ -22,6 +22,10 @@ over-reports.
   cpu_baseline  the CPU oracle (oracle/, a restatement of the Ceres 1.14 path the reference runs) on the host cores
 
 --impl reference times that CPU oracle alone, with all host threads, on the same workload/metric.
+
+--dump-outputs DIR writes, after the timed steps, what the timed path returned to its caller in its last step (see
+dump_outputs) as DIR/<name>.npy.  The workloads are generated from fixed seeds, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import hashlib
@@ -39,6 +43,14 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 ITERS_PER_SOLVE = 5
+
+# --dump-outputs: a parameter vector of up to DUMP_MAX_FULL entries (32 MB in float64) is written whole; a larger one
+# (cfg5 has 12M) as a sample of DUMP_SAMPLE entries drawn with DUMP_SEED, beside their positions, 32 MB in all
+DUMP_MAX_FULL = 1 << 22
+DUMP_SAMPLE = 1 << 21
+DUMP_SEED = 0xBAD0
+DUMP_ROW_FIELDS = ("cost", "cost_change", "gradient_max_norm", "step_norm", "trust_region_radius", "linear_solver_iterations",
+                   "step_is_successful")
 
 # name -> (description, model, generator kwargs, rcs solver)
 WORKLOADS = {
@@ -129,6 +141,7 @@ class Job:
             self.blocks = {"n_cameras": pr.n_cam, "n_frames": pr.n_time, "n_markers": pr.n_marker, "n_marker_obs": pr.n_mobs,
                            "n_corner_obs": 4 * pr.n_mobs}
             self.sharded = "frames"
+        self.lo, self.hi = sh.lo, sh.hi
         self.params = self.local[-1]
         self.h2d = sum(np.asarray(a).nbytes for a in self.local[1:]) + pr.intr.nbytes
 
@@ -154,6 +167,14 @@ class Job:
         else:
             n_time, ti, ci, mi, obs8, _ = self.local
             P.set_model_b(pr.n_cam, n_time, pr.n_marker, ti, ci, mi, obs8, pr.intr, pr.marker_side, True)
+
+    def merge(self, shard_results):
+        """(lo, hi, rank-local parameter vector) of every rank -> the parameter vector of the whole problem."""
+        from realsensecalibration_b200 import sharding
+        pr = self.pr
+        if self.model == "A":
+            return sharding.merge_model_a(pr.n_cam, pr.n_pt, shard_results)
+        return sharding.merge_model_b(pr.n_cam, pr.n_time, pr.n_marker, shard_results)
 
     def oracle_solver(self, O):
         # the rule BA_RCS_AUTO applies (ba_cuda.cu, kDenseAutoMaxN): dense Cholesky up to dimension 1536, PCG above
@@ -239,12 +260,20 @@ def run_steps(P, opts, k):
             P.solve_begin(opts)
             P.solve_iterate(n)
             out = P.solve_end()
+        check_steps(out[1], n)
         done += n
     return out
 
 
+def check_steps(rows, n):
+    """A solve that stopped before its n LM iterations would make K / time over-report: refuse to count it."""
+    if len(rows) != n + 1:   # row 0 is the initial evaluation
+        raise RuntimeError("a solve asked for %d LM iterations ran %d: the timed steps would not be --steps" % (n, len(rows) - 1))
+
+
 def oracle_steps(job, k, threads):
-    """The reference arm: the CPU oracle on the same workload, same restart rule; returns (seconds, rows)."""
+    """The reference arm: the CPU oracle on the same workload, same restart rule; returns (seconds, rows, summary, x) of
+    the last solve."""
     from oracle import oracle_py as O
     o = O.default_options()
     o.function_tolerance = 0.0; o.parameter_tolerance = 0.0; o.gradient_tolerance = 0.0
@@ -253,10 +282,32 @@ def oracle_steps(job, k, threads):
         n = min(ITERS_PER_SOLVE, k - done)
         o.max_num_iterations = n
         t0 = time.perf_counter()
-        _, s, rows = job.oracle_solve(O, o, threads)
+        x, s, rows = job.oracle_solve(O, o, threads)
         t += time.perf_counter() - t0
+        check_steps(rows, n)
         done += n
-    return t, rows, s
+    return t, rows, s, x
+
+
+def dump_outputs(out_dir, x, summary, rows):
+    """--dump-outputs: what the timed path handed its caller after its last step, one float64 .npy file per array --
+    the parameter vector (what ba_cuda_get_parameters returns, or the oracle's solution on --impl reference; a fixed,
+    seeded sample of it above DUMP_MAX_FULL entries, with the positions of the sample in parameters_index), the progress rows of the last solve (row 0 is the cost it started
+    from) and its final cost."""
+    os.makedirs(out_dir, exist_ok=True)
+    x = np.asarray(x, np.float64)
+    arrays = {}
+    if x.size <= DUMP_MAX_FULL:
+        arrays["parameters"] = x
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(x.size, DUMP_SAMPLE, replace=False))
+        arrays["parameters"] = x[idx]
+        arrays["parameters_index"] = idx.astype(np.float64)
+    for k in DUMP_ROW_FIELDS:
+        arrays[k] = np.array([r[k] for r in rows], np.float64)
+    arrays["final_cost"] = np.array([summary.final_cost], np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def config_of(job, name, n_gpus, rcs_solver, rcs_dim):
@@ -290,7 +341,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-jacobian", action="store_true", help="skip the standalone residual+Jacobian kernel timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -306,7 +360,9 @@ def main():
         threads = host_threads()
         if W > 0:
             oracle_steps(job, min(W, 1), threads)
-        secs, rows, osum = oracle_steps(job, K, threads)
+        secs, rows, osum, x = oracle_steps(job, K, threads)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, x, osum, rows)
         v = K / secs
         print(json.dumps({
             "impl": "reference", "metric": metric, "value": v, "unit": unit, "n_gpus": a.gpus, "steps": K, "warmup": W,
@@ -375,6 +431,15 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = K / (ms * 1e-3)
+    if a.dump_outputs:
+        # now, before the passes below overwrite the problem's parameters
+        x = P.get_parameters()
+        if dist is not None:
+            got = [None] * world
+            dist.all_gather_object(got, (job.lo, job.hi, x))
+            x = job.merge(got)
+        if rank == 0:
+            dump_outputs(a.dump_outputs, x, summary, rows)
 
     # the same K steps once more with an event pair around every kernel (costs a few us per launch, which is why it is
     # not the timed pass): per-kernel device times for the roofline and the kernel shares
@@ -477,7 +542,7 @@ def main():
         from oracle import oracle_py as O
         threads = host_threads()
         kc = min(K, ITERS_PER_SOLVE)
-        secs, _, osum = oracle_steps(job, kc, threads)
+        secs, _, osum, _ = oracle_steps(job, kc, threads)
         cpu = {"value": kc / secs, "unit": unit, "cores": threads, "kind": "port",
                "threads_from": "CPU affinity of the process, passed to the oracle's num_threads clauses",
                "final_cost": float(osum.final_cost),

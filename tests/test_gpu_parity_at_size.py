@@ -7,6 +7,8 @@ an inexact Newton step: with the CG iteration count fixed on both sides (pcg_min
 Ceres' Q-based stopping rule a flip by one CG iteration moves the step, so that trace is held to 1e-7 while the counts agree."""
 import json
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -16,6 +18,8 @@ from realsensecalibration_b200 import abi, cuda
 from tests import helpers as H
 
 pytestmark = pytest.mark.gpu
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "synth_traces.json")) as f:
     TRACES = json.load(f)
@@ -90,3 +94,31 @@ def test_bal_configurations_at_full_size(gpu, name):
     worst = _compare(rows, tr["rows"], 1e-7, name)
     print("%s: worst relative cost difference: %.2e with %d CG iterations per solve, %.2e with the stopping rule" %
           (name, worst_fixed, tr["fixed_cg"], worst))
+
+
+def test_bench_dumps_the_last_step_of_the_timed_solves(gpu, oracle, tmp_path):
+    # bench.py --dump-outputs: 7 steps are one solve of 5 LM iterations and one of 2; the dump is what a caller of the same
+    # 7 steps receives (bit for bit: the library has no floating-point atomics) and the oracle's 2-iteration solve to the
+    # parity tolerances
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--workload", "small", "--steps", "7", "--warmup", "2",
+                        "--no-cpu-baseline", "--no-e2e", "--no-jacobian", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 7
+    arrays = {p.stem: np.load(p) for p in out.glob("*.npy")}
+    assert sorted(arrays) == sorted(("parameters", "final_cost") + bench.DUMP_ROW_FIELDS)
+    job = bench.Job("small", 0, 1)
+    job.set_model(gpu)
+    gpu.set_parameters(job.params)
+    gpu.save_parameters()
+    s, rows = bench.run_steps(gpu, bench.bench_options(cuda, profile=False), 7)
+    assert np.array_equal(arrays["parameters"], gpu.get_parameters()) and np.array_equal(arrays["cost"], [r["cost"] for r in rows])
+    assert arrays["final_cost"][0] == s.final_cost
+    o = oracle.default_options()
+    o.function_tolerance = 0.0; o.parameter_tolerance = 0.0; o.gradient_tolerance = 0.0; o.max_num_iterations = 2
+    xo, so, rows_o = job.oracle_solve(oracle, o, bench.host_threads())
+    assert len(rows_o) == 3
+    for a, b in zip(arrays["cost"], rows_o):
+        assert H.rel(a, b["cost"]) <= 1e-10, (a, b)
+    assert np.abs(arrays["parameters"] - xo).max() < 1e-7
