@@ -48,7 +48,8 @@ typedef enum ba_status {
   BA_ERR_NCCL = -4,
   BA_ERR_OUT_OF_MEMORY = -5,
   BA_ERR_NO_DEVICE = -6,
-  BA_ERR_UNSUPPORTED = -7
+  BA_ERR_UNSUPPORTED = -7,
+  BA_ERR_RANK_DEFICIENT = -8  /* ba_cuda_covariance: the normal equations at x are singular */
 } ba_status;
 
 /* How the reduced camera system (RCS) is solved; replaces
@@ -275,6 +276,26 @@ int ba_cuda_get_iterations(ba_cuda_problem* p, ba_cuda_iteration* rows, int cap)
  *   Model B: residuals 8/mobs; jac 144/mobs = [d r/d cam (8x6) | d r/d frame (8x6) | d r/d marker (8x6)],
  *            blocks the functor does not take are zero. */
 int ba_cuda_eval(ba_cuda_problem* p, double* cost, double* residuals, double* jac);
+
+/* ceres::Covariance (apply_loss_function = true) over the free parameters at the CURRENT parameters, Model B only:
+ * C = (J^T J)^-1, J = the Jacobian the solver sees (rows scaled by Ceres' Corrector when options->loss_function is set;
+ * NULL options = ba_cuda_options_init defaults; only loss_function / loss_scale are read, and profile_kernels for the
+ * per-kernel timing).  Not multiplied by a residual variance (Ceres does not either).  Outputs, any of them may be NULL:
+ *   cov_kept   [6(n_cam+n_marker)]^2 row-major, blocks in parameter order [cameras | markers] (camera c at row 6c, marker m
+ *              at 6(n_cam+m)); rows / columns of blocks that are not parameters (camera 0, marker 0 under fix_marker0,
+ *              blocks no observation references) are 0.  Exactly symmetric.
+ *   cov_frames n_time x 36: the 6x6 diagonal block of every frame pose (0 for unobserved frames)
+ *   smallest_pivot_ratio: min_k d_k / max_k S_kk over the parameter rows of the Jacobi-scaled reduced system S = L D L^T
+ *              (a diagnostic of its conditioning; 0 when the factorisation meets a pivot <= 0)
+ * The rank test is a pivot test, not Ceres' eigenvalue criterion: BA_ERR_RANK_DEFICIENT (cov_kept and cov_frames untouched,
+ * smallest_pivot_ratio written) when E^T E of a frame pose does not factor or smallest_pivot_ratio <= min_pivot_ratio
+ * (<= 0: 1e-12), e.g. the 6-dimensional gauge freedom of frame poses against marker poses when no marker is fixed.
+ * BA_ERR_STATE without a model and parameters or inside an open solve; BA_ERR_UNSUPPORTED for Model A (every camera is
+ * free: J^T J always has a 7-dimensional gauge null space and this ABI has no constant blocks), for world size > 1 and
+ * for a reduced system above 1536 (256 cameras + markers).  Uses the solve's workspace: call it between solves. */
+int ba_cuda_covariance(ba_cuda_problem* p, const ba_cuda_options* options, double min_pivot_ratio,
+                       double* cov_kept, double* cov_frames, double* smallest_pivot_ratio);
+
 /* device time (ms, CUDA events) of the last ba_cuda_eval / ba_cuda_reprojection_error kernel */
 /* ---- the numeric part of the correspondence stage that runs just before the path (SURVEY.md 8 f1).  ArUco detection and
  *      solvePnP (EPnP) stay with OpenCV; these are the pose algebra and corner construction around them, in the conventions of

@@ -10,6 +10,8 @@ CONVERGENCE, NO_CONVERGENCE, FAILURE = 0, 1, 2
 UNIQUE_ID_BYTES = 128
 PATH_GENERIC, PATH_FUSED_TILES, PATH_FUSED_STRIPS, PATH_RIG = 0, 1, 2, 3
 LOSS_NONE, LOSS_HUBER, LOSS_CAUCHY = 0, 1, 2
+(ERR_INVALID_ARGUMENT, ERR_CUDA, ERR_STATE, ERR_NCCL, ERR_OUT_OF_MEMORY, ERR_NO_DEVICE, ERR_UNSUPPORTED,
+ ERR_RANK_DEFICIENT) = range(-1, -9, -1)
 
 
 class Options(C.Structure):

@@ -23,6 +23,7 @@
 #include "ba_strip_a.cuh"
 #include "ba_exchange.cuh"
 #include "ba_rig.cuh"
+#include "ba_cov.cuh"
 
 using namespace ba;
 
@@ -72,13 +73,15 @@ enum Family { F_JAC = 0, F_SCHUR, F_SOLVE, F_UPDATE, F_COST, F_COLL, F_COUNT };
 // one entry per kernel (family member) of the solve path; names are what ba_cuda_get_kernel_stats() reports
 enum KT {
   KT_TABLES = 0, KT_JAC, KT_COST, KT_FOBS, KT_EM, KT_INCW, KT_DOBS, KT_ECHOL, KT_INCY, KT_FINC, KT_PAIRS, KT_SEGFIN,
-  KT_ASSEMBLE, KT_RCS, KT_BACKSUB, KT_MODELCOST, KT_CANDIDATE, KT_GRADNORM, KT_FOLD, KT_MISC, KT_FA_P1, KT_FA_RED, KT_FA_P2, KT_FA_P1L, KT_RIG, KT_COUNT
+  KT_ASSEMBLE, KT_RCS, KT_BACKSUB, KT_MODELCOST, KT_CANDIDATE, KT_GRADNORM, KT_FOLD, KT_MISC, KT_FA_P1, KT_FA_RED, KT_FA_P2, KT_FA_P1L, KT_RIG,
+  KT_COV_LINV, KT_COV_INV, KT_COV_FRAMES, KT_COUNT
 };
 const char* const kKtName[KT_COUNT] = {
   "k1_tables", "k1_residual_jacobian", "k5_cost", "k2_fobs_partial", "k2_e_normal", "k2_inc_w", "k2_dobs_partial",
   "k2_e_cholesky", "k2_inc_y", "k2_finc_partial", "k2_pairs_partial", "k2_seg_final", "k2_assemble", "k3_rcs_solve",
   "k4_backsub", "k4_model_cost", "k4_candidate", "k4_gradient_norm", "fold_partials", "misc",
-  "k1k2_fused_pass1", "k2_reduce_items", "k4k5_fused_pass2", "k1_fused_pass1_light", "rig_lm_whole_loop"};
+  "k1k2_fused_pass1", "k2_reduce_items", "k4k5_fused_pass2", "k1_fused_pass1_light", "rig_lm_whole_loop",
+  "cov_l_inverse", "cov_inverse_kept", "cov_frames"};
 }  // namespace
 
 struct LmState {  // TrustRegionMinimizer's loop variables, kept between ba_cuda_solve_iterate() calls
@@ -477,10 +480,11 @@ int eval_gradient_and_jacobian(ba_cuda_problem* p, bool first, bool jacobi_scali
   return run_gradient_norms_f(p);
 }
 
-// LevenbergMarquardtStrategy::ComputeStep + SchurEliminator + dense Cholesky + BackSubstitute + the model cost
-// change and the candidate point.  scal[S_RADIUS] must hold the trust-region radius.
-template <int RD, int DE, int GE, int NSLOT>
-int compute_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
+// SchurEliminator for the LM diagonal of the radius in scal[S_RADIUS]: frame / point blocks factored (Lb, zb), Yt, and
+// the reduced camera system with its rhs (Sd | rhs, or Sb | rhs for PCG).  Leaves the F_SOLVE family open: the caller's
+// solve of the system belongs to it.  The covariance runs it with radius = +inf, i.e. without LM diagonal.
+template <int RD, int DE>
+int schur_complement(ba_cuda_problem* p, const ba_cuda_options& opt) {
   const Structure& S = p->S;
   const int64_t n = p->n_rcs();
   const double* radius = p->scal.p + S_RADIUS;
@@ -520,17 +524,29 @@ int compute_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
     fam_end(p, F_COLL);
   }
   fam_begin(p, F_SOLVE);
-  if (pcg) {
+  if (pcg)
     BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_bsr, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->R.diag.p, p->HG.p, NV_F, p->vsum(), 6, radius,
               opt.min_lm_diagonal, opt.max_lm_diagonal, p->Sb.p, p->rhs.p);
+  else
+    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_dense, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->HG.p, NV_F, p->vsum(), 6, radius, opt.min_lm_diagonal,
+              opt.max_lm_diagonal, n, p->Sd.p, p->rhs.p);
+  return BA_OK;
+}
+
+// LevenbergMarquardtStrategy::ComputeStep + SchurEliminator + dense Cholesky + BackSubstitute + the model cost
+// change and the candidate point.  scal[S_RADIUS] must hold the trust-region radius.
+template <int RD, int DE, int GE, int NSLOT>
+int compute_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
+  const Structure& S = p->S;
+  const int64_t n = p->n_rcs();
+  BA_TRY((schur_complement<RD, DE>(p, opt)));
+  if (p->solver == BA_RCS_PCG) {
     {
       LaunchScope scope(p, KT_RCS);
       BA_TRY(launch_pcg(p->pcg, p->R, p->Sb.p, p->rhs.p, p->yf.p, p->status.p, opt, p->st));
     }
     BA_CUDA_TRY(cudaMemcpyAsync(&p->h_pcg_iters, p->pcg.iters.p, sizeof(int), cudaMemcpyDeviceToHost, p->st));
   } else {
-    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_dense, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->HG.p, NV_F, p->vsum(), 6, radius, opt.min_lm_diagonal,
-              opt.max_lm_diagonal, n, p->Sd.p, p->rhs.p);
     LaunchScope scope(p, KT_RCS);
     BA_TRY(dense_solve(p, n));
   }
@@ -1573,6 +1589,58 @@ void reset_problem(ba_cuda_problem* p) {
   new (&p->S) Structure();
 }
 
+// ba_cuda_covariance after its checks: Model B, one rank, n <= kDenseAutoMaxN, p->loss set (ba_cov.cuh has the algebra).
+int covariance_impl(ba_cuda_problem* p, const ba_cuda_options& opt, double min_pivot_ratio, double* cov_kept, double* cov_frames,
+                    double* smallest_pivot_ratio) {
+  const Structure& S = p->S;
+  const int n = (int)p->n_rcs();
+  cudaStream_t st = p->st;
+  BA_TRY(prepare_solver(p, opt));   // opt.rcs_solver is BA_RCS_DENSE_CHOLESKY: Sd exists
+  BA_TRY(ensure_generic_workspace(p));
+  BA_TRY((eval_gradient_and_jacobian<8, 6, 32>(p, true, true)));
+  BA_LAUNCH(p, KT_MISC, k_cov_unit_unused<6>, grid_for(S.ne + S.nf, 256), 256, 0, S.ne, S.e_ptr.p, p->ME.p, S.nf, p->f_act_ptr.p, p->HG.p);
+  const double no_lm_diagonal_radius = INFINITY;   // D^2 = clamp(diag) / radius = 0 exactly
+  BA_CUDA_TRY(cudaMemcpyAsync(p->scal.p + S_RADIUS, &no_lm_diagonal_radius, sizeof(double), cudaMemcpyHostToDevice, st));
+  BA_TRY((schur_complement<8, 6>(p, opt)));
+  DVec<double> diag, X, Sig, Ck, Cf;
+  BA_TRY(diag.alloc(n + 1)); BA_TRY(X.alloc_zero((size_t)n * n, st)); BA_TRY(Sig.alloc((size_t)n * n)); BA_TRY(Ck.alloc((size_t)n * n));
+  BA_TRY(Cf.alloc((size_t)S.ne * 36));
+  BA_LAUNCH(p, KT_MISC, k_cov_save_diag, grid_for(n, 256), 256, 0, n, p->Sd.p, diag.p);
+  {
+    LaunchScope scope(p, KT_RCS);
+    BA_TRY(launch_chol_blocked(p->cholb, n, p->Sd.p, p->rhs.p, p->yf.p, p->status.p, p->device, st));
+  }
+  BA_LAUNCH(p, KT_MISC, k_cov_pivot_ratio, 1, 1024, 0, n, p->Sd.p, diag.p, p->f_act_ptr.p, diag.p + n);
+  BA_LAUNCH(p, KT_COV_LINV, k_cov_linv, (n + CV_NB - 1) / CV_NB, CV_THREADS, 0, n, p->Sd.p, X.p);
+  const int nt = (n + CV_TB - 1) / CV_TB;
+  BA_LAUNCH(p, KT_COV_INV, k_cov_inverse, nt * (nt + 1) / 2, CV_THREADS, 0, n, X.p, p->sf.p, p->f_act_ptr.p, Sig.p, Ck.p);
+  fam_end(p, F_SOLVE);
+  if (S.ne > 0) {
+    const size_t smem = cov_frames_smem(6, S.nf);
+    if (smem > 48 * 1024) BA_CUDA_TRY(cudaFuncSetAttribute(k_cov_frames<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    BA_LAUNCH(p, KT_COV_FRAMES, k_cov_frames<6>, (unsigned)S.ne, CV_THREADS, smem, S.ne, S.e_ptr.p, S.einc_ptr, S.inc_f, p->Yt.p, p->Lb.p,
+              p->se.p, Sig.p, n, Cf.p);
+  }
+  BA_CUDA_TRY(cudaGetLastError());
+  double ratio = 0.0;
+  BA_CUDA_TRY(cudaMemcpyAsync(&ratio, diag.p + n, sizeof(double), cudaMemcpyDeviceToHost, st));
+  BA_CUDA_TRY(cudaMemcpyAsync(p->h_status, p->status.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+  BA_CUDA_TRY(cudaStreamSynchronize(st));
+  fam_collect(p);
+  const int status = *p->h_status;
+  if (status & 2) ratio = 0.0;   // the factorisation stopped at a pivot <= 0
+  if (smallest_pivot_ratio) *smallest_pivot_ratio = ratio;
+  if (status & 1) return fail(BA_ERR_RANK_DEFICIENT, "ba_cuda_covariance: E^T E of a frame pose is not positive definite");
+  const double thr = min_pivot_ratio > 0.0 ? min_pivot_ratio : 1e-12;
+  if (!(ratio > thr))
+    return fail(BA_ERR_RANK_DEFICIENT, "ba_cuda_covariance: the reduced system is rank deficient (smallest pivot / largest diagonal entry "
+                "%.3e <= %.3e)", ratio, thr);
+  if (cov_kept) BA_CUDA_TRY(cudaMemcpyAsync(cov_kept, Ck.p, sizeof(double) * (size_t)n * n, cudaMemcpyDeviceToHost, st));
+  if (cov_frames && S.ne > 0) BA_CUDA_TRY(cudaMemcpyAsync(cov_frames, Cf.p, sizeof(double) * (size_t)S.ne * 36, cudaMemcpyDeviceToHost, st));
+  BA_CUDA_TRY(cudaStreamSynchronize(st));
+  return BA_OK;
+}
+
 }  // namespace
 
 // =======================================================================================
@@ -2041,6 +2109,11 @@ static double algorithmic_bytes(const ba_cuda_problem* p, int kt) {
     case KT_FA_P1L: return nb * (184.0 + 116.0 + 64.0) + ne * (24.0 + 72.0) + nf * (80.0 + 216.0);
     // pass 2 = K4 (152 B/obs + 72 B/point read, 24 B/point + 48 B/camera written) + cost-only evaluation (24 B/obs)
     case KT_FA_P2: return nb * (152.0 + 24.0) + ne * (72.0 + 24.0 + 24.0) + nf * (48.0 + 80.0);
+    // covariance (ba_cov.cuh), n = 6 nf: L^-1 reads L and writes X (lower triangles); X^T X reads X and writes two full n x n
+    // matrices; the frame blocks read Yt, Lb, se and S^-1 once (every later read of S^-1 is an L2 hit) and write 36 per frame
+    case KT_COV_LINV: return 8.0 * (36.0 * nf * nf);
+    case KT_COV_INV: return 20.0 * (36.0 * nf * nf);
+    case KT_COV_FRAMES: return ninc * 288.0 + ne * (288.0 + 48.0 + 288.0) + 8.0 * (36.0 * nf * nf);
     default: return 0.0;
   }
 }
@@ -2128,6 +2201,37 @@ int ba_cuda_eval(ba_cuda_problem* p, double* cost, double* residuals, double* ja
   return BA_OK;
 }
 
+int ba_cuda_covariance(ba_cuda_problem* p, const ba_cuda_options* options, double min_pivot_ratio, double* cov_kept,
+                       double* cov_frames, double* smallest_pivot_ratio) {
+  if (!p) return fail(BA_ERR_INVALID_ARGUMENT, "NULL problem");
+  if (p->model < 0 || !p->params_set) return fail(BA_ERR_STATE, "set_model_b and set_parameters must be called before ba_cuda_covariance");
+  // the covariance overwrites the Jacobian, the scaling and the Schur workspace the open solve works on
+  if (p->lm.began && p->lm.go) return fail(BA_ERR_STATE, "ba_cuda_covariance between ba_cuda_solve_begin and the end of the solve");
+  if (p->model != 1)
+    return fail(BA_ERR_UNSUPPORTED, "ba_cuda_covariance: Model A is not supported (every camera is free, so J^T J has the 7-dimensional "
+                "gauge null space of a similarity transform, and there are no constant blocks to remove it)");
+  if (p->world > 1) return fail(BA_ERR_UNSUPPORTED, "ba_cuda_covariance runs on one GPU (world size %d)", p->world);
+  if (p->n_rcs() > kDenseAutoMaxN)
+    return fail(BA_ERR_UNSUPPORTED, "ba_cuda_covariance: reduced system of dimension %lld is above %lld", (long long)p->n_rcs(),
+                (long long)kDenseAutoMaxN);
+  ba_cuda_options opt;
+  ba_cuda_options_init(&opt);
+  if (options) {
+    opt.loss_function = options->loss_function; opt.loss_scale = options->loss_scale;
+    opt.profile_kernels = options->profile_kernels;
+  }
+  if (opt.loss_function < BA_LOSS_NONE || opt.loss_function > BA_LOSS_CAUCHY || (opt.loss_function != BA_LOSS_NONE && !(opt.loss_scale > 0.0)))
+    return fail(BA_ERR_INVALID_ARGUMENT, "loss_function %d with scale %g", opt.loss_function, opt.loss_scale);
+  opt.rcs_solver = BA_RCS_DENSE_CHOLESKY;
+  BA_TRY(use_device(p));
+  const bool profile = p->profile;
+  p->loss = LossSpec{opt.loss_function, opt.loss_scale};
+  p->profile = opt.profile_kernels != 0;
+  const int rc = covariance_impl(p, opt, min_pivot_ratio, cov_kept, cov_frames, smallest_pivot_ratio);
+  p->loss = LossSpec{0, 1.0};
+  p->profile = profile;
+  return rc;
+}
 
 int ba_cuda_reprojection_error(ba_cuda_problem* p, double* sum_half_sq, double* rms_per_coord) {
   if (!p) return fail(BA_ERR_INVALID_ARGUMENT, "NULL problem");

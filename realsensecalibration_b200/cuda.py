@@ -24,12 +24,16 @@ EXPORTS = [
     "ba_cuda_project_points_error", "ba_cuda_model_b_outputs", "ba_cuda_solve_begin", "ba_cuda_solve_iterate",
     "ba_cuda_solve_end", "ba_cuda_set_stream", "ba_cuda_get_kernel_stats", "ba_cuda_num_launches", "ba_cuda_reset_stats",
     "ba_cuda_save_parameters", "ba_cuda_restore_parameters", "ba_cuda_project_points_error_rt",
-    "ba_cuda_release_cached_memory", "ba_cuda_marker_corners", "ba_cuda_compose_poses",
+    "ba_cuda_release_cached_memory", "ba_cuda_marker_corners", "ba_cuda_compose_poses", "ba_cuda_covariance",
 ]
 
 
 class BAError(RuntimeError):
-    pass
+    """A ba_cuda_* call failed; `code` is its ba_status (abi.ERR_*)."""
+
+    def __init__(self, message, code=None):
+        super().__init__(message)
+        self.code = code
 
 
 def build():
@@ -55,9 +59,13 @@ def lib():
     return _LIB
 
 
+def _error(rc):
+    return BAError("ba_cuda error %d: %s" % (rc, lib().ba_cuda_last_error().decode()), rc)
+
+
 def _check(rc):
     if rc != 0:
-        raise BAError("ba_cuda error %d: %s" % (rc, lib().ba_cuda_last_error().decode()))
+        raise _error(rc)
 
 
 def default_options():
@@ -132,7 +140,7 @@ class Problem:
                                          ti.ctypes, ci.ctypes, mi.ctypes, ob.ctypes, K.ctypes, C.c_double(marker_side),
                                          C.c_int32(1), C.c_int32(int(fix_marker0))))
         self.model, self.n_obs = "B", int(ti.shape[0])
-        self.n_cam = n_cam
+        self.n_cam, self.n_time, self.n_marker = n_cam, n_time, n_marker
 
     def num_parameters(self):
         return int(lib().ba_cuda_num_parameters(self._h))
@@ -206,6 +214,24 @@ class Problem:
         _check(lib().ba_cuda_eval(self._h, C.byref(cost), None if res is None else res.ctypes.data_as(C.c_void_p),
                                   None if jac is None else jac.ctypes.data_as(C.c_void_p)))
         return cost.value, res, jac
+
+    def covariance(self, options=None, min_pivot_ratio=0.0):
+        """ceres::Covariance of the free parameters at the current parameters (Model B; include/ba_cuda.h):
+        (cov_kept [6(C+M), 6(C+M)] in parameter order [cameras | markers], cov_frames [T, 6, 6], smallest_pivot_ratio).
+        A rank-deficient problem raises BAError with code abi.ERR_RANK_DEFICIENT and the ratio as `smallest_pivot_ratio`."""
+        kept = frames = None   # no Model B: the library refuses the call (BA_ERR_STATE / BA_ERR_UNSUPPORTED) and writes nothing
+        if self.model == "B":
+            nk = 6 * (self.n_cam + self.n_marker)
+            kept = np.zeros((nk, nk)); frames = np.zeros((self.n_time, 6, 6))
+        ratio = C.c_double(0.0)
+        rc = lib().ba_cuda_covariance(self._h, None if options is None else C.byref(options), C.c_double(min_pivot_ratio),
+                                      None if kept is None else kept.ctypes.data_as(C.c_void_p),
+                                      None if frames is None else frames.ctypes.data_as(C.c_void_p), C.byref(ratio))
+        if rc != 0:
+            err = _error(rc)
+            err.smallest_pivot_ratio = ratio.value
+            raise err
+        return kept, frames, ratio.value
 
     def last_kernel_ms(self):
         return float(lib().ba_cuda_last_kernel_ms(self._h))

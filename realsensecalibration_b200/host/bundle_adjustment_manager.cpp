@@ -47,7 +47,7 @@ BAManager::BAManager(const std::map<std::string, cv::Mat>& camera_intrinsics_map
 // (camera_idx == 0, marker_idx == 0) is done inside ba_cuda_set_model_b (fix_cam0 = 1, fix_marker0 = Main/Test2);
 // intrinsics are looked up by SERIAL_NUMBERS[camera_idx] exactly as manager.cpp:34,47,64,78 do; the solver
 // options are Ceres' defaults with DENSE_SCHUR and progress to stdout (manager.cpp:90-92).
-void BAManager::StartBA() {
+std::vector<double> BAManager::Intrinsics4() const {
   const int C = bal_problem.num_cameras();
   if ((int)serial_numbers_.size() < C) Die("BAManager: fewer serial numbers than cameras");
   std::vector<double> intr(4 * (size_t)C);
@@ -58,6 +58,12 @@ void BAManager::StartBA() {
     intr[4 * c + 0] = K.at<double>(0, 0); intr[4 * c + 1] = K.at<double>(1, 1);   // fx, fy   (bundle_adjustment.h:66-67)
     intr[4 * c + 2] = K.at<double>(0, 2); intr[4 * c + 3] = K.at<double>(1, 2);   // ppx, ppy (bundle_adjustment.h:68-69)
   }
+  return intr;
+}
+
+void BAManager::StartBA() {
+  const int C = bal_problem.num_cameras();
+  const std::vector<double> intr = Intrinsics4();
   ba_cuda_problem* p = nullptr;
   auto check = [&](int rc, const char* what) {
     if (rc != BA_OK) { std::string m = std::string(what) + ": " + ba_cuda_last_error(); ba_cuda_destroy(p); Die(m); }
@@ -92,6 +98,34 @@ void BAManager::StartBA() {
        << "\n\nMinimizer iterations  " << summary_.num_iterations << "\nSuccessful steps      " << summary_.num_successful_steps
        << "\nUnsuccessful steps    " << summary_.num_unsuccessful_steps << "\n\nTime (s): total " << summary_.total_time_s
        << "\nTermination: " << kTerm[summary_.termination_type] << " (" << kWhy[summary_.termination_reason] << ")\n" << endl;
+}
+
+int BAManager::Covariance(std::vector<double>* camera_cov, std::vector<double>* frame_cov) {
+  const int C = bal_problem.num_cameras(), M = bal_problem.num_markers();
+  const std::vector<double> intr = Intrinsics4();
+  const size_t nk = 6 * ((size_t)C + M);
+  std::vector<double> kept(nk * nk), frames(36 * (size_t)bal_problem.num_times());
+  ba_cuda_options options;
+  ba_cuda_options_init(&options);
+  options.loss_function = loss_function_; options.loss_scale = loss_scale_;   // the loss StartBA() solved with
+  ba_cuda_problem* p = nullptr;
+  int rc = ba_cuda_create(&p, device_);
+  if (rc == BA_OK)
+    rc = ba_cuda_set_model_b(p, C, bal_problem.num_times(), M, bal_problem.num_observations(), bal_problem.time_index(),
+                             bal_problem.camera_index(), bal_problem.marker_index(), bal_problem.observations(), intr.data(),
+                             bal_problem.marker_side(), 1, fix_base_marker_ ? 1 : 0);
+  if (rc == BA_OK) rc = ba_cuda_set_parameters(p, bal_problem.parameters(), bal_problem.num_parameters());
+  if (rc == BA_OK) rc = ba_cuda_covariance(p, &options, 0.0, kept.data(), frames.data(), nullptr);
+  ba_cuda_destroy(p);
+  if (rc != BA_OK) return rc;
+  if (camera_cov) {   // GetCovarianceBlock(camera_c, camera_c)
+    camera_cov->assign(36 * (size_t)C, 0.0);
+    for (int c = 0; c < C; ++c)
+      for (int a = 0; a < 6; ++a)
+        for (int b = 0; b < 6; ++b) (*camera_cov)[36 * (size_t)c + 6 * a + b] = kept[(6 * (size_t)c + a) * nk + 6 * c + b];
+  }
+  if (frame_cov) frame_cov->swap(frames);
+  return BA_OK;
 }
 
 // bundle_adjustment_manager.cpp:98-175: Camera_Transform.xml (R<i> 3x3, t<i> 3x1, 17 digits), the inverse pose

@@ -31,6 +31,7 @@ class BAManager {
   ba_cuda_summary summary_{};
   std::vector<ba_cuda_iteration> iterations_;
   void Load();
+  std::vector<double> Intrinsics4() const;   // fx, fy, ppx, ppy per camera, looked up by serial number
 
  public:
   BAManager(const std::map<std::string, cv::Mat>& camera_intrinsics_map, const std::map<std::string, cv::Mat>& dist_coeffs_map);
@@ -51,6 +52,11 @@ class BAManager {
             const Config& config);
   const ba_cuda_summary& summary() const { return summary_; }
   const std::vector<ba_cuda_iteration>& iterations() const { return iterations_; }
+  // ceres::Covariance + GetCovarianceBlock after StartBA(), at the solved parameters and with its loss: the 6x6 covariance
+  // of every camera pose (CAMERAS x 36, row-major; camera 0 is not a parameter: zeros) and of every frame pose
+  // (num_times x 36).  Either output may be NULL.  Returns BA_OK or the ba_status of ba_cuda_covariance
+  // (BA_ERR_RANK_DEFICIENT when the problem has a gauge freedom, e.g. no marker fixed); the message is ba_cuda_last_error().
+  int Covariance(std::vector<double>* camera_cov, std::vector<double>* frame_cov);
   BALProblem& problem() { return bal_problem; }
 };
 

@@ -1,9 +1,12 @@
 // main_calibration_ba.cpp -- the bundle-adjustment stage of Main_Calibration's main() (main.cpp:35-43) on the
 // files the earlier stages leave behind, driven through the source-compatible host classes:
 //   BAManager(intrinsics, dist) -> StartBA() -> Write() -> ReprojectionCheck::Reproject(...)
-// usage: ba_main_calibration <Common dir> <output dir> [test1 | test2]
+// usage: ba_main_calibration <Common dir> <output dir> [test1 | test2 | covariance]
+// covariance: the hongo run, followed by one line per camera with the standard deviations of its pose parameters
+// (rvec, tvec; per unit of pixel noise) from ceres::Covariance's counterpart (BAManager::Covariance).
 // Everything before it in the reference's main() (image capture, ArUco detection, solvePnP) is out of scope; the
 // detected corners Reproject needs are the observations stored in correspondence.txt.
+#include <cmath>
 #include <cstdio>
 #include <iostream>
 
@@ -71,5 +74,14 @@ int main(int argc, char** argv) {
   std::cout << "Average Reprojection Error per One Coordinate: " << r.rms_per_coordinate << std::endl;
   std::printf("summary: iterations %d initial %.15e final %.15e reprojection %.12e rms %.8f\n", ba_manager.summary().num_iterations,
               ba_manager.summary().initial_cost, ba_manager.summary().final_cost, r.reprojection_error, r.rms_per_coordinate);
+  if (argc > 3 && std::string(argv[3]) == "covariance") {
+    std::vector<double> cam;
+    if (ba_manager.Covariance(&cam, nullptr) != BA_OK) { std::cerr << ba_cuda_last_error() << std::endl; return 1; }
+    for (int c = 0; c < pb.num_cameras(); ++c) {
+      std::printf("covariance: camera %d sd", c);
+      for (int k = 0; k < 6; ++k) std::printf(" %.6e", std::sqrt(cam[36 * (size_t)c + 7 * k]));
+      std::printf("\n");
+    }
+  }
   return 0;
 }
