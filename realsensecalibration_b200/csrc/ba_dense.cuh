@@ -1,8 +1,8 @@
 // ba_dense.cuh -- K3a: dense Cholesky solve of a rig-sized reduced camera system in ONE CTA.
 // Replaces Ceres' DenseSchurComplementSolver -> Eigen LLT (options.linear_solver_type = DENSE_SCHUR,
-// bundle_adjustment_manager.cpp:91).  For n <= 160 the whole matrix lives in shared memory
-// (n^2 * 8 B <= 205 KB of the 227 KB a CTA may use on sm_100a); larger systems are factored in
-// place in global memory (L2 resident) by the same code.
+// bundle_adjustment_manager.cpp:91).  The whole matrix lives in shared memory, so n <= 160
+// (n^2 * 8 B <= 205 KB of the 227 KB a CTA may use on sm_100a); larger systems go to ba_dense_blocked.cuh.
+// Only the lower triangle and the diagonal of S are read.
 #pragma once
 #include "ba_util.cuh"
 
@@ -10,17 +10,16 @@ namespace ba {
 
 constexpr int CHOL_SMEM_MAX_N = 160;
 
-template <bool SMEM>
+// status |= 2 (and y = 0) if a pivot is not positive, |= 4 if the solution is not finite.
 __global__ void __launch_bounds__(1024)
-k_chol_solve(int n, double* __restrict__ S, const double* __restrict__ rhs, double* __restrict__ y, int* status) {
+k_chol_solve(int n, const double* __restrict__ S, const double* __restrict__ rhs, double* __restrict__ y, int* status) {
   extern __shared__ double sh[];
-  double* A = SMEM ? sh : S;
-  double* col = SMEM ? sh + (size_t)n * n : sh;
+  double* A = sh;
+  double* col = sh + (size_t)n * n;
   double* bv = col + n;
   const int tid = threadIdx.x, nt = blockDim.x;
   const int lane = tid & 31, warp = tid >> 5, nw = nt >> 5;
-  if (SMEM)
-    for (int i = tid; i < n * n; i += nt) A[i] = S[i];
+  for (int i = tid; i < n * n; i += nt) A[i] = S[i];
   for (int i = tid; i < n; i += nt) bv[i] = rhs[i];
   bool bad = false;
   for (int j = 0; j < n; ++j) {
@@ -71,19 +70,13 @@ k_chol_solve(int n, double* __restrict__ S, const double* __restrict__ rhs, doub
   }
 }
 
-inline int launch_chol_solve(int n, double* S, const double* rhs, double* y, int* status, cudaStream_t st) {
-  if (n <= CHOL_SMEM_MAX_N) {
-    const size_t smem = ((size_t)n * n + 2 * (size_t)n) * sizeof(double);
-    // the opt-in limit belongs to the device the stream runs on; setting it costs microseconds, a process-wide
-    // "done" flag would leave a second GPU without it
-    if (smem > 48 * 1024) BA_CUDA_TRY(cudaFuncSetAttribute(k_chol_solve<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    k_chol_solve<true><<<1, 1024, smem, st>>>(n, S, rhs, y, status);
-  } else {
-    const size_t smem = 2 * (size_t)n * sizeof(double);
-    if (smem > 200 * 1024) return fail(BA_ERR_UNSUPPORTED, "dense RCS of dimension %d is too large for the single-CTA solver", n);
-    if (smem > 48 * 1024) BA_CUDA_TRY(cudaFuncSetAttribute(k_chol_solve<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    k_chol_solve<false><<<1, 1024, smem, st>>>(n, S, rhs, y, status);
-  }
+inline int launch_chol_solve(int n, const double* S, const double* rhs, double* y, int* status, cudaStream_t st) {
+  if (n > CHOL_SMEM_MAX_N) return fail(BA_ERR_UNSUPPORTED, "dense RCS of dimension %d is too large for the single-CTA solver", n);
+  const size_t smem = ((size_t)n * n + 2 * (size_t)n) * sizeof(double);
+  // the opt-in limit belongs to the device the stream runs on; setting it costs microseconds, a process-wide
+  // "done" flag would leave a second GPU without it
+  if (smem > 48 * 1024) BA_CUDA_TRY(cudaFuncSetAttribute(k_chol_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  k_chol_solve<<<1, 1024, smem, st>>>(n, S, rhs, y, status);
   BA_CUDA_TRY(cudaGetLastError());
   return BA_OK;
 }

@@ -659,7 +659,8 @@ __global__ void __launch_bounds__(RIG_THREADS, 1) k_rig_lm(const RigParams P) {
 }
 
 // The same factorisation as a kernel of its own: the dense reduced-system solve of the multi-kernel pipeline for n <= RIG_MAX_N
-// (S row-major n x n in HBM, not modified).  status bit 1 is raised when a pivot is not positive.
+// (S row-major n x n in HBM, not modified; only its lower triangle and diagonal are read).  As the other dense solvers:
+// status |= 2 and y = 0 when a pivot is not positive, status |= 4 when the solution is not finite.
 __global__ void __launch_bounds__(RIG_THREADS, 1)
 k_ldlt_small(int n, const double* __restrict__ Sg, const double* __restrict__ rhs_g, double* __restrict__ y, int* status) {
   extern __shared__ __align__(16) double dsm[];
@@ -678,7 +679,10 @@ k_ldlt_small(int n, const double* __restrict__ Sg, const double* __restrict__ rh
   if (!rig_ldlt_solve(S, n, ld, rhs, invd, tacc, blk, y, nullptr)) {
     for (int i = threadIdx.x; i < n; i += RIG_THREADS) y[i] = 0.0;
     if (threadIdx.x == 0) atomicOr(status, 2);
+    return;
   }
+  for (int i = threadIdx.x; i < n; i += RIG_THREADS)   // rhs holds the solution (rig_ldlt_solve ends on a barrier)
+    if (!isfinite(rhs[i])) atomicOr(status, 4);
 }
 
 inline size_t rig_smem_bytes(int n) { return sizeof(double) * (((size_t)n + 1) * (n | 1) + 2 * (size_t)n + 66); }

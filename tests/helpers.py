@@ -3,7 +3,7 @@ import os
 
 import numpy as np
 
-from realsensecalibration_b200 import formats as F
+from realsensecalibration_b200 import abi, formats as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden", "reference_common")
@@ -68,3 +68,46 @@ def check_test2_golden(x, tol=5e-14):
 
 def rel(a, b):
     return abs(a - b) / max(abs(b), 1e-300)
+
+
+# ---- the numpy twin of the normal equations (test_covariance.py, test_dense_solvers.py) ----
+def _rho1(loss, a, s):
+    if loss == abi.LOSS_HUBER:
+        return np.where(s > a * a, a / np.sqrt(np.maximum(s, 1e-300)), 1.0)
+    if loss == abi.LOSS_CAUCHY:
+        return 1.0 / (1.0 + s / (a * a))
+    return np.ones_like(s)
+
+
+def normal_equations(oracle, pb, intr, side, fix0, x, loss=abi.LOSS_NONE, scale=1.0):
+    """J^T J as a dense [6 nblk]^2 matrix over the blocks [cameras | frames | markers] and the mask of the free blocks.
+    Accumulated block-wise (np.add.at over the 3 x 3 block pairs of every marker observation)."""
+    C, T, M = pb.n_cam, pb.n_time, pb.n_marker
+    _, res, jac = oracle.eval_model_b(pb, intr, side, fix0, params=x)
+    w = np.sqrt(_rho1(loss, scale, (res ** 2).sum(axis=1)))
+    J = jac.reshape(-1, 3, 8, 6).transpose(0, 2, 1, 3) * w[:, None, None, None]   # [obs, row, block, col]
+    blk = np.stack([pb.cam_idx, C + pb.time_idx, C + T + pb.marker_idx], 1)
+    nb = C + T + M
+    Hb = np.zeros((nb, nb, 6, 6))
+    for a in range(3):
+        for b in range(3):
+            np.add.at(Hb, (blk[:, a], blk[:, b]), np.einsum("nri,nrj->nij", J[:, :, a], J[:, :, b]))
+    free = np.zeros(nb, bool)
+    free[blk.ravel()] = True
+    free[0] = False                       # camera 0 is never a parameter block
+    if fix0:
+        free[C + T] = False               # marker 0 under the Main dispatch
+    return Hb.transpose(0, 2, 1, 3).reshape(6 * nb, 6 * nb), free
+
+
+def reduced_system(oracle, pb, intr, side, fix0, x):
+    """The Jacobi-scaled reduced camera system over the free kept blocks (the frames eliminated), without an LM diagonal."""
+    C, T = pb.n_cam, pb.n_time
+    Hd, free = normal_equations(oracle, pb, intr, side, fix0, x)
+    s = 1.0 / (1.0 + np.sqrt(np.diag(Hd)))
+    Hs = Hd * s[:, None] * s[None, :]
+    fs = np.repeat(free, 6)
+    is_frame = np.zeros(Hd.shape[0], bool)
+    is_frame[6 * C:6 * (C + T)] = True
+    e, f = np.flatnonzero(fs & is_frame), np.flatnonzero(fs & ~is_frame)
+    return Hs[np.ix_(f, f)] - Hs[np.ix_(f, e)] @ np.linalg.solve(Hs[np.ix_(e, e)], Hs[np.ix_(e, f)])
