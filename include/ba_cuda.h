@@ -269,6 +269,36 @@ int ba_cuda_solve_end(ba_cuda_problem* p, ba_cuda_summary* summary);
 /* rows of the progress table; returns the number of rows available (>= 0) */
 int ba_cuda_get_iterations(ba_cuda_problem* p, ba_cuda_iteration* rows, int cap);
 
+/* k independent solves of this problem's structure in one launch, one CTA each (Monte Carlo runs under fresh corner
+ * noise, multi-start against the planar-marker pose ambiguity).  The model, intrinsics, marker side and fixed-block dispatch
+ * are the problem's; one `options` applies to every instance (NULL = ba_cuda_options_init defaults; the loss is validated as
+ * ba_cuda_solve_begin validates it).  Arguments:
+ *   params        k x n_params, caller layout of ba_cuda_set_parameters: instance i starts from params + i n_params and
+ *                 its solution is written there.  Blocks that are not parameters or that no observation references come
+ *                 back as given.
+ *   observations  NULL (every instance uses the model's own observations) or k x (2 n_obs | 8 n_mobs), each instance in the
+ *                 caller's order of ba_cuda_set_model_a / ba_cuda_set_model_b.
+ *   summaries     k, or NULL.
+ *   rows          k x rows_cap, or NULL: instance i's first rows_cap rows of the progress table at rows + i rows_cap;
+ *                 summaries[i].num_iterations is its full count.
+ * Instance i gives what ba_cuda_set_model_* with its observations, ba_cuda_set_parameters(params + i n_params) and
+ * ba_cuda_solve(options) give, bit for bit in the parameters, in every row field except iteration_time_s and in every
+ * summary field except total_time_s (here the host wall clock of the whole call) and the ms_* timings (0 here).  Results do
+ * not depend on k or on which CTA ran an instance.  A numerical failure of an instance (e.g. a non-finite start ->
+ * BA_REASON_INITIAL_EVALUATION_FAILED) is reported in its summary and the call still returns BA_OK, as ba_cuda_solve does.
+ * minimizer_progress_to_stdout is not honoured.
+ * The problem is left as it was: its parameters, progress rows, summary and saved snapshot are untouched; the batch works
+ * in per-instance buffers of its own (DESIGN.md 3.2c gives the bytes per instance).
+ * BA_ERR_UNSUPPORTED wherever ba_cuda_solve would not run on BA_PATH_RIG for size or configuration: a reduced system above
+ * 160, more than 8192 residual rows, PCG, force_generic_path, world size > 1.  BA_ERR_STATE without a model or inside an open
+ * solve; BA_ERR_INVALID_ARGUMENT for k < 1, NULL params or rows with rows_cap < 1; BA_ERR_OUT_OF_MEMORY when the
+ * per-instance buffers cannot be allocated (the problem stays usable).  The launches are counted in
+ * ba_cuda_get_kernel_stats as "rig_lm_batch"; the work runs on the problem's stream and the call returns after a
+ * synchronise. */
+int ba_cuda_solve_batch(ba_cuda_problem* p, const ba_cuda_options* options, int32_t k, double* params,
+                        const double* observations, ba_cuda_summary* summaries, ba_cuda_iteration* rows,
+                        int32_t rows_cap);
+
 /* One residual + Jacobian evaluation at the current parameters (test hook and
  * the "residual+Jacobian Mobs/s" measurement).  Outputs may be NULL.  Layouts,
  * in the caller's observation order:

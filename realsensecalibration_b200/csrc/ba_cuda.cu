@@ -12,6 +12,7 @@
 #include <atomic>
 #include <chrono>
 #include <cmath>
+#include <cstddef>
 #include <string>
 
 #include "ba_dense.cuh"
@@ -74,14 +75,14 @@ enum Family { F_JAC = 0, F_SCHUR, F_SOLVE, F_UPDATE, F_COST, F_COLL, F_COUNT };
 enum KT {
   KT_TABLES = 0, KT_JAC, KT_COST, KT_FOBS, KT_EM, KT_INCW, KT_DOBS, KT_ECHOL, KT_INCY, KT_FINC, KT_PAIRS, KT_SEGFIN,
   KT_ASSEMBLE, KT_RCS, KT_BACKSUB, KT_MODELCOST, KT_CANDIDATE, KT_GRADNORM, KT_FOLD, KT_MISC, KT_FA_P1, KT_FA_RED, KT_FA_P2, KT_FA_P1L, KT_RIG,
-  KT_COV_LINV, KT_COV_INV, KT_COV_FRAMES, KT_COUNT
+  KT_COV_LINV, KT_COV_INV, KT_COV_FRAMES, KT_RIG_BATCH, KT_COUNT
 };
 const char* const kKtName[KT_COUNT] = {
   "k1_tables", "k1_residual_jacobian", "k5_cost", "k2_fobs_partial", "k2_e_normal", "k2_inc_w", "k2_dobs_partial",
   "k2_e_cholesky", "k2_inc_y", "k2_finc_partial", "k2_pairs_partial", "k2_seg_final", "k2_assemble", "k3_rcs_solve",
   "k4_backsub", "k4_model_cost", "k4_candidate", "k4_gradient_norm", "fold_partials", "misc",
   "k1k2_fused_pass1", "k2_reduce_items", "k4k5_fused_pass2", "k1_fused_pass1_light", "rig_lm_whole_loop",
-  "cov_l_inverse", "cov_inverse_kept", "cov_frames"};
+  "cov_l_inverse", "cov_inverse_kept", "cov_frames", "rig_lm_batch"};
 }  // namespace
 
 struct LmState {  // TrustRegionMinimizer's loop variables, kept between ba_cuda_solve_iterate() calls
@@ -1018,12 +1019,16 @@ void lm_read_gradient(ba_cuda_problem* p) {
 
 // ---- the rig-size path (ba_rig.cuh): one CTA runs the whole loop ---------------------------------------------
 int ensure_generic_workspace(ba_cuda_problem* p);
+// the size and configuration test of the one-CTA path (ba_cuda_solve and ba_cuda_solve_batch); `solver` is the resolved
+// rcs_solver, `max_rows` the residual-row limit
+bool rig_fits(const ba_cuda_problem* p, int solver, bool force_generic_path, int64_t max_rows) {
+  const int64_t rows = p->S.nb * (p->model == 0 ? 2 : 8);
+  return p->world == 1 && !force_generic_path && solver == BA_RCS_DENSE_CHOLESKY && p->n_rcs() <= RIG_MAX_N && rows <= max_rows;
+}
 bool rig_eligible(const ba_cuda_problem* p, const ba_cuda_options& opt) {
   const bool on = env_int("BA_RIG", 0, 1, 1) != 0;   // read per solve: tests run both machines in one process
-  const int64_t rows = p->S.nb * (p->model == 0 ? 2 : 8);
   const int64_t max_rows = env_int("BA_RIG_MAX_ROWS", 0, 1 << 30, (int)RIG_MAX_ROWS);   // tuning aid (profiles/tools/rig_crossover.py)
-  return on && p->world == 1 && !opt.force_generic_path && p->solver == BA_RCS_DENSE_CHOLESKY && p->n_rcs() <= RIG_MAX_N &&
-         rows <= max_rows;
+  return on && rig_fits(p, p->solver, opt.force_generic_path != 0, max_rows);
 }
 
 template <int RD, int DE, int GE, int NSLOT>
@@ -1570,6 +1575,166 @@ __global__ void k_corners_b(int64_t nb, const int32_t* __restrict__ perm, const 
   o[0] = r[0] + Tt[18]; o[1] = r[1] + Tt[19]; o[2] = r[2] + Tt[20];
 }
 
+// ---- ba_cuda_solve_batch: K solves of one structure in one launch, one CTA each (ba_rig.cuh, k_rig_lm_batch) ---------
+// instance i's observation j (structure order) is row i * n + perm[j] of the caller's k x n rows: with this map one
+// k_gather_uv launch over all k * n rows puts every instance into structure order
+__global__ void k_batch_perm(const int32_t* __restrict__ perm, int64_t n, int64_t k, int32_t* __restrict__ out) {
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t < n * k) out[t] = (int32_t)((t / n) * n + perm[t % n]);
+}
+
+// the arrays of one instance's slice of the batch workspace
+enum RigBatchArray {
+  RB_XE = 0, RB_XF, RB_XE_C, RB_XF_C, RB_SE, RB_SF, RB_TAB_F, RB_TAB_E, RB_TABC_F, RB_TABC_E,
+  RB_RES, RB_JE, RB_JF0, RB_JF1, RB_ME, RB_HG, RB_WT, RB_QACC, RB_LB, RB_ZB, RB_YT, RB_VB, RB_PACC, RB_VSUM, RB_YF, RB_YE, RB_COUNT
+};
+// caller parameter layout <-> the instance slices: (caller offset, slice array, slice offset, count) per segment
+struct ParamSegment { int64_t src, dst_arr, dst, count; };
+int param_segments(const ba_cuda_problem* p, ParamSegment seg[3]) {
+  const int64_t C = p->n_cam;
+  if (p->model == 0) {
+    seg[0] = {0, RB_XF, 0, 6 * C};
+    seg[1] = {6 * C, RB_XE, 0, 3 * p->n_pt};
+    return 2;
+  }
+  const int64_t T = p->n_time, M = p->n_marker;
+  seg[0] = {0, RB_XF, 0, 6 * C};
+  seg[1] = {6 * C, RB_XE, 0, 6 * T};
+  seg[2] = {6 * (C + T), RB_XF, 6 * C, 6 * M};
+  return 3;
+}
+
+template <int RD, int DE, int GE, int NSLOT>
+int rig_batch_run(ba_cuda_problem* p, const ba_cuda_options& opt, int32_t k, double* params, const double* observations,
+                  ba_cuda_summary* summaries, ba_cuda_iteration* rows, int32_t rows_cap) {
+  const double t_start = now_s();
+  const Structure& S = p->S;
+  const cudaStream_t st = p->st;
+  const int n = (int)p->n_rcs();
+  constexpr int NU = DE * (DE + 1) / 2;
+  constexpr bool MB = RD == 8;
+  // one region per instance; every array starts on a 32-byte boundary (J, uv and obs8 are read as double2)
+  int64_t len[RB_COUNT] = {};
+  len[RB_XE] = len[RB_XE_C] = len[RB_SE] = len[RB_ZB] = len[RB_YE] = S.ne * DE;
+  len[RB_XF] = len[RB_XF_C] = len[RB_SF] = len[RB_VSUM] = S.nf * 6;
+  len[RB_YF] = n;
+  len[RB_TAB_F] = len[RB_TABC_F] = S.nf * TAB;
+  len[RB_TAB_E] = len[RB_TABC_E] = MB ? S.ne * TAB : 0;
+  len[RB_RES] = S.nb * RD; len[RB_JE] = S.nb * RD * DE; len[RB_JF0] = S.nb * RD * 6; len[RB_JF1] = MB ? S.nb * RD * 6 : 0;
+  len[RB_ME] = S.ne * (NU + DE); len[RB_HG] = S.nf * NV_F; len[RB_WT] = MB ? S.ninc * 36 : 0; len[RB_QACC] = MB ? (int64_t)S.ndest * 36 : 0;
+  len[RB_LB] = S.ne * DE * DE; len[RB_YT] = S.ninc * DE * 6; len[RB_VB] = S.ninc * 6; len[RB_PACC] = (int64_t)S.ndest * 36;
+  int64_t off[RB_COUNT];
+  RigBatch B;
+  std::memset(&B, 0, sizeof(B));
+  for (int j = 0; j < RB_COUNT; ++j) { off[j] = B.stride; B.stride += (len[j] + 3) / 4 * 4; }
+  // rows one launch can record per instance: a solve records at most max_num_iterations + 1
+  const int64_t R = std::max<int64_t>(1, std::min<int64_t>(RIG_ROWS_CAP, (int64_t)opt.max_num_iterations + 1));
+  B.rows_stride = R;
+  DVec<double> ws, obs_raw, obs;
+  DVec<RigState> states;
+  DVec<ba_cuda_iteration> drows;
+  DVec<int32_t> perm;
+  BA_TRY(ws.alloc_zero((size_t)k * B.stride, st));   // zeroed: the blocks no step touches read as they would in a fresh problem
+  BA_TRY(states.alloc(k));
+  BA_TRY(drows.alloc((size_t)k * R));
+  const size_t D = sizeof(double);
+  ParamSegment seg[3];
+  const int nseg = param_segments(p, seg);
+  for (int s = 0; s < nseg; ++s)
+    if (seg[s].count)
+      BA_CUDA_TRY(cudaMemcpy2DAsync(ws.p + off[seg[s].dst_arr] + seg[s].dst, D * B.stride, params + seg[s].src, D * p->n_params,
+                                    D * seg[s].count, k, cudaMemcpyHostToDevice, st));
+  if (observations) {
+    const int width = MB ? 8 : 2;
+    const int64_t rows_all = (int64_t)k * S.nb;
+    BA_TRY(obs_raw.upload(observations, (size_t)rows_all * width, st));
+    BA_TRY(perm.alloc(rows_all)); BA_TRY(obs.alloc((size_t)rows_all * width));
+    BA_LAUNCH(p, KT_MISC, k_batch_perm, grid_for(rows_all, 256), 256, 0, S.perm.p, S.nb, (int64_t)k, perm.p);
+    BA_LAUNCH(p, KT_MISC, k_gather_uv, grid_for(rows_all * width, 256), 256, 0, obs_raw.p, perm.p, rows_all, width, obs.p);
+    BA_CUDA_TRY(cudaGetLastError());
+    B.obs = obs.p; B.obs_stride = S.nb * width;
+  }
+  // what rig_run passes
+  RigParams P;
+  std::memset(&P, 0, sizeof(P));
+  P.nb = S.nb; P.ne = S.ne; P.nf = S.nf; P.ninc = S.ninc; P.ndest = S.ndest; P.n = n; P.ld = n | 1;
+  P.ob_e = S.ob_e.p; P.ob_f0 = S.ob_f0.p; P.ob_f1 = S.ob_f1.p; P.ob_cam = p->ob_cam.p; P.e_ptr = S.e_ptr.p;
+  P.inc_e = S.inc_e; P.inc_f = S.inc_f; P.einc_ptr = S.einc_ptr; P.incobs_ptr = S.incobs_ptr.p; P.incobs = S.incobs.p;
+  P.finc_ptr = S.finc_ptr.p; P.fobs_ptr = S.fobs_ptr.p; P.finc = S.finc.p; P.fobs = S.fobs.p;
+  P.dest_fa = S.dest_fa.p; P.dest_fb = S.dest_fb.p; P.dpair_ptr = S.dpair_ptr.p; P.pairs = S.pairs.p;
+  P.dobs_ptr = S.dobs_ptr.p; P.dobs = S.dobs.p; P.f_act_ptr = p->f_act_ptr.p;
+  P.uv = p->uv.p; P.obs8 = p->obs8.p; P.intr_f = p->intr_f.p; P.half_side = p->half_side;
+  // instance 0's arrays; the kernel moves them B.stride doubles further per instance
+  double** const arr[RB_COUNT] = {&P.xe, &P.xf, &P.xe_c, &P.xf_c, &P.se, &P.sf, &P.tab_f, &P.tab_e, &P.tabc_f, &P.tabc_e,
+                                  &P.RES, &P.JE, &P.JF0, &P.JF1, &P.ME, &P.HG, &P.Wt, &P.Qacc, &P.Lb, &P.zb, &P.Yt, &P.vb,
+                                  &P.Pacc, &P.vsum, &P.yf, &P.ye};
+  for (int j = 0; j < RB_COUNT; ++j) *arr[j] = ws.p + off[j];
+  P.state = states.p; P.rows = drows.p;
+  P.opt = opt; P.loss = LossSpec{opt.loss_function, opt.loss_scale};
+  P.init.radius = opt.initial_trust_region_radius; P.init.decrease_factor = 2.0; P.init.go = 1;
+  const size_t smem = rig_smem_bytes(n);
+  BA_CUDA_TRY(cudaFuncSetAttribute(k_rig_lm_batch<RD, DE, GE, NSLOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rig_smem_bytes(RIG_MAX_N)));
+  std::vector<RigState> hst(k);
+  std::vector<int32_t> base(k, 0);
+  std::vector<double> cost0(k, 0.0);
+  std::vector<ba_cuda_iteration> hrows;
+  bool running = true;
+  for (int64_t launch = 0; running; ++launch) {   // a solve longer than RIG_ROWS_CAP rows continues in the next launch, as in rig_run
+    P.begin = launch == 0 ? 1 : 0;
+    P.max_new = RIG_ROWS_CAP - P.begin;
+    BA_LAUNCH(p, KT_RIG_BATCH, (k_rig_lm_batch<RD, DE, GE, NSLOT>), (unsigned)k, RIG_THREADS, smem, P, B);
+    BA_CUDA_TRY(cudaGetLastError());
+    BA_CUDA_TRY(cudaMemcpyAsync(hst.data(), states.p, sizeof(RigState) * k, cudaMemcpyDeviceToHost, st));
+    if (launch == 0)   // row 0's cost is the summary's initial_cost
+      BA_CUDA_TRY(cudaMemcpy2DAsync(cost0.data(), D, reinterpret_cast<const char*>(drows.p) + offsetof(ba_cuda_iteration, cost),
+                                    sizeof(ba_cuda_iteration) * R, D, k, cudaMemcpyDeviceToHost, st));
+    // the rows of this launch start at row launch * RIG_ROWS_CAP of every instance still running: fetch those the caller keeps
+    const int64_t first = launch * RIG_ROWS_CAP;
+    const int64_t cnt = rows ? std::min<int64_t>(R, rows_cap - first) : 0;
+    if (cnt > 0) {
+      hrows.resize((size_t)k * cnt);
+      BA_CUDA_TRY(cudaMemcpy2DAsync(hrows.data(), sizeof(ba_cuda_iteration) * cnt, drows.p, sizeof(ba_cuda_iteration) * R,
+                                    sizeof(ba_cuda_iteration) * cnt, k, cudaMemcpyDeviceToHost, st));
+    }
+    BA_CUDA_TRY(cudaStreamSynchronize(st));
+    fam_collect(p);
+    running = false;
+    for (int32_t i = 0; i < k; ++i) {
+      const int64_t fresh = hst[i].n_rows - base[i];
+      for (int64_t r = 0; r < std::min(fresh, cnt); ++r)
+        if (base[i] + r < rows_cap) rows[(int64_t)i * rows_cap + base[i] + r] = hrows[(size_t)i * cnt + r];
+      base[i] = hst[i].n_rows;
+      running = running || hst[i].go != 0;
+    }
+  }
+  for (int s = 0; s < nseg; ++s)
+    if (seg[s].count)
+      BA_CUDA_TRY(cudaMemcpy2DAsync(params + seg[s].src, D * p->n_params, ws.p + off[seg[s].dst_arr] + seg[s].dst, D * B.stride,
+                                    D * seg[s].count, k, cudaMemcpyDeviceToHost, st));
+  BA_CUDA_TRY(cudaStreamSynchronize(st));
+  if (summaries) {   // rig_run + lm_end + ba_cuda_solve_end, per instance
+    const double total = now_s() - t_start;
+    for (int32_t i = 0; i < k; ++i) {
+      const RigState& s = hst[i];
+      ba_cuda_summary& Z = summaries[i];
+      std::memset(&Z, 0, sizeof(Z));
+      Z.termination_type = s.term_type; Z.termination_reason = s.term_reason;
+      Z.num_iterations = s.n_rows;
+      Z.num_successful_steps = s.n_success; Z.num_unsuccessful_steps = s.n_unsuccess;
+      Z.rcs_solver_used = BA_RCS_DENSE_CHOLESKY;
+      Z.rcs_dim = (int32_t)(6 * p->n_active_f_global);
+      Z.num_jacobian_evaluations = s.n_jac; Z.num_cost_evaluations = s.n_solves; Z.num_linear_solves = s.n_solves;
+      Z.num_residuals = p->nb_global * RD;
+      Z.num_free_parameters = p->n_active_e_global * DE + p->n_active_f_global * 6;
+      Z.initial_cost = s.n_rows > 0 ? cost0[i] : s.x_cost;
+      Z.final_cost = s.x_cost;
+      Z.total_time_s = total;
+      Z.path_used = BA_PATH_RIG;
+    }
+  }
+  return BA_OK;
+}
+
 void reset_problem(ba_cuda_problem* p) {
   p->model = -1;
   p->params_set = false;
@@ -2072,6 +2237,42 @@ int ba_cuda_solve(ba_cuda_problem* p, const ba_cuda_options* options, ba_cuda_su
   int32_t finished = 0;
   BA_TRY(ba_cuda_solve_iterate(p, INT32_MAX, &finished));
   return ba_cuda_solve_end(p, summary);
+}
+
+int ba_cuda_solve_batch(ba_cuda_problem* p, const ba_cuda_options* options, int32_t k, double* params, const double* observations,
+                        ba_cuda_summary* summaries, ba_cuda_iteration* rows, int32_t rows_cap) {
+  if (!p) return fail(BA_ERR_INVALID_ARGUMENT, "NULL problem");
+  if (p->model < 0) return fail(BA_ERR_STATE, "set_model_* must be called before ba_cuda_solve_batch");
+  if (p->lm.began && p->lm.go) return fail(BA_ERR_STATE, "ba_cuda_solve_batch between ba_cuda_solve_begin and the end of the solve");
+  if (k < 1 || !params || (rows && rows_cap < 1))
+    return fail(BA_ERR_INVALID_ARGUMENT, "ba_cuda_solve_batch: k = %d, params %s, rows_cap = %d", k, params ? "set" : "NULL", rows_cap);
+  ba_cuda_options opt;
+  if (options) opt = *options; else ba_cuda_options_init(&opt);
+  if (opt.loss_function < BA_LOSS_NONE || opt.loss_function > BA_LOSS_CAUCHY || (opt.loss_function != BA_LOSS_NONE && !(opt.loss_scale > 0.0)))
+    return fail(BA_ERR_INVALID_ARGUMENT, "loss_function %d with scale %g", opt.loss_function, opt.loss_scale);
+  int solver = opt.rcs_solver;   // as prepare_solver resolves it
+  if (solver == BA_RCS_AUTO) solver = p->n_rcs() <= kDenseAutoMaxN ? BA_RCS_DENSE_CHOLESKY : BA_RCS_PCG;
+  if (solver != BA_RCS_DENSE_CHOLESKY && solver != BA_RCS_PCG) return fail(BA_ERR_INVALID_ARGUMENT, "unknown rcs_solver %d", opt.rcs_solver);
+  if (!rig_fits(p, solver, opt.force_generic_path != 0, RIG_MAX_ROWS))
+    return fail(BA_ERR_UNSUPPORTED, "ba_cuda_solve_batch takes rig-size problems only (reduced system %lld <= %d, residual rows %lld <= %lld, "
+                "dense rcs_solver, force_generic_path = 0, one GPU): got %lld, %lld, rcs_solver %d, force_generic_path %d, world size %d",
+                (long long)p->n_rcs(), RIG_MAX_N, (long long)(p->S.nb * (p->model == 0 ? 2 : 8)), (long long)RIG_MAX_ROWS,
+                (long long)p->n_rcs(), (long long)(p->S.nb * (p->model == 0 ? 2 : 8)), solver, opt.force_generic_path, p->world);
+  if (observations && (int64_t)k * p->S.nb > (int64_t)INT32_MAX)
+    return fail(BA_ERR_UNSUPPORTED, "ba_cuda_solve_batch: %d instances of %lld observations are too many for one call", k, (long long)p->S.nb);
+  BA_TRY(use_device(p));
+  BA_TRY(ensure_generic_workspace(p));   // the pair lists of the structure
+  const bool profile = p->profile;
+  p->profile = opt.profile_kernels != 0;
+  const int rc = p->model == 0 ? rig_batch_run<2, 3, 1, 1>(p, opt, k, params, observations, summaries, rows, rows_cap)
+                               : rig_batch_run<8, 6, 32, 2>(p, opt, k, params, observations, summaries, rows, rows_cap);
+  p->profile = profile;
+  if (rc != BA_OK) {   // the per-instance buffers are gone; the problem's own were never touched
+    cudaStreamSynchronize(p->st);
+    p->pending.clear();
+    p->ev_next = 0;
+  }
+  return rc;
 }
 
 int ba_cuda_set_stream(ba_cuda_problem* p, void* cuda_stream) {

@@ -25,6 +25,7 @@ EXPORTS = [
     "ba_cuda_solve_end", "ba_cuda_set_stream", "ba_cuda_get_kernel_stats", "ba_cuda_num_launches", "ba_cuda_reset_stats",
     "ba_cuda_save_parameters", "ba_cuda_restore_parameters", "ba_cuda_project_points_error_rt",
     "ba_cuda_release_cached_memory", "ba_cuda_marker_corners", "ba_cuda_compose_poses", "ba_cuda_covariance",
+    "ba_cuda_solve_batch",
 ]
 
 
@@ -170,6 +171,38 @@ class Problem:
         rows = (Iteration * max(n, 1))()
         lib().ba_cuda_get_iterations(self._h, rows, C.c_int(n))
         return s, [rows[i].as_dict() for i in range(n)]
+
+    def solve_batch(self, params, observations=None, options=None, rows_cap=None):
+        """k independent solves of this problem's structure in one launch (ba_cuda_solve_batch, include/ba_cuda.h).
+
+        params: [k, n_params] starts.  observations: None (the model's own) or [k, n_obs, 2] (Model A) / [k, n_mobs, 8]
+        (Model B) in the order given to set_model_*.  rows_cap: progress rows kept per instance (None: all of them,
+        options.max_num_iterations + 1; 0: none).  Returns (solutions [k, n_params], k summaries, k row lists), the summaries
+        and rows as `solve` returns them."""
+        opts = options or default_options()
+        x = np.array(params, dtype=np.float64, order="C", copy=True)   # the library writes the solutions into it
+        obs = None
+        if self.model is not None:   # without a model the library refuses the call (BA_ERR_STATE)
+            if x.ndim != 2 or x.shape[1] != self.num_parameters():
+                raise ValueError("params must have shape [k, %d], got %s" % (self.num_parameters(), x.shape))
+            if observations is not None:
+                obs = np.ascontiguousarray(observations, np.float64)
+                width = 2 if self.model == "A" else 8
+                if obs.shape != (x.shape[0], self.n_obs, width):
+                    raise ValueError("observations must have shape [%d, %d, %d], got %s" % (x.shape[0], self.n_obs, width, obs.shape))
+        k = x.shape[0] if x.ndim == 2 else 1
+        if rows_cap is None:
+            rows_cap = max(1, int(opts.max_num_iterations) + 1)
+        summaries = (Summary * max(k, 1))()
+        rows = (Iteration * (k * rows_cap))() if rows_cap > 0 and k > 0 else None
+        _check(lib().ba_cuda_solve_batch(self._h, C.byref(opts), C.c_int32(k), x.ctypes.data_as(C.c_void_p),
+                                         None if obs is None else obs.ctypes.data_as(C.c_void_p), summaries,
+                                         rows, C.c_int32(rows_cap)))
+        out_rows = []
+        for i in range(k):
+            n = min(summaries[i].num_iterations, rows_cap) if rows is not None else 0
+            out_rows.append([rows[i * rows_cap + r].as_dict() for r in range(n)])
+        return x, [summaries[i] for i in range(k)], out_rows
 
     def _rows(self):
         n = lib().ba_cuda_get_iterations(self._h, None, C.c_int(0))
