@@ -526,10 +526,10 @@ int schur_complement(ba_cuda_problem* p, const ba_cuda_options& opt) {
   }
   fam_begin(p, F_SOLVE);
   if (pcg)
-    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_bsr, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->R.diag.p, p->HG.p, NV_F, p->vsum(), 6, radius,
+    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_bsr<>, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->R.diag.p, p->HG.p, NV_F, p->vsum(), 6, radius,
               opt.min_lm_diagonal, opt.max_lm_diagonal, p->Sb.p, p->rhs.p);
   else
-    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_dense, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->HG.p, NV_F, p->vsum(), 6, radius, opt.min_lm_diagonal,
+    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_dense<>, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->HG.p, NV_F, p->vsum(), 6, radius, opt.min_lm_diagonal,
               opt.max_lm_diagonal, n, p->Sd.p, p->rhs.p);
   return BA_OK;
 }
@@ -592,7 +592,7 @@ FaParams fa_params(ba_cuda_problem* p, const ba_cuda_options& opt) {
   P.citem_begin = F.cams.item_begin.p; P.citem_end = F.cams.item_end.p; P.cent = F.cams.ent.p;
   P.xe = p->xe.p; P.se = p->se.p; P.tab_f = p->tab_f.p; P.radius = p->scal.p + S_RADIUS;
   P.min_diag = opt.min_lm_diagonal; P.max_diag = opt.max_lm_diagonal;
-  P.partP = F.partP.p; P.partC = F.partC.p; P.Lz = F.Lz.p; P.se_out = p->se.p;
+  P.partP = F.red_pairs.part.p; P.partC = F.red_cams.part.p; P.Lz = F.Lz.p; P.se_out = p->se.p;
   P.cost_partial = p->fa_part.p; P.g2_partial = p->fa_part.p + nt; P.gmax_partial = p->fa_part.p + 2 * nt;
   P.yf = p->yf.p; P.tabc_f = p->tabc_f.p; P.xe_c = p->xe_c.p;
   P.mcc_partial = p->fa_part.p + 3 * nt; P.x2_partial = p->fa_part.p + 4 * nt; P.d2_partial = p->fa_part.p + 5 * nt;
@@ -620,106 +620,30 @@ int fa_set_smem_attr(ba_cuda_problem* p) {
   return BA_OK;
 }
 
-int fa_reduce(ba_cuda_problem* p, bool cams, bool pairs) {
-  const Structure& S = p->S;
-  FusedA& F = p->FA;
-  if (cams) {
-    const ItemSet& I = F.cams;
-    if (I.red_ch.n > 0)
-      BA_LAUNCH(p, KT_FA_RED, (k_reduce_items<FA_NVC>), grid_for(I.red_ch.n, 4), 128, 0, I.red_ch.n, I.red_ch.ch, I.red_ch.seg.p, I.red_ch.begin.p,
-                I.tgt_ptr.p, I.red_items.p, F.partC.p, F.red1C.p);
-    BA_LAUNCH(p, KT_FA_RED, (k_reduce_final<FA_NVC>), grid_for(S.nf, 4), 128, 0, (int)S.nf, I.red_ch.seg_first.p, F.red1C.p, F.camacc.p);
-  }
-  if (pairs) {
-    const ItemSet& I = F.pairs;
-    if (I.red_ch.n > 0)
-      BA_LAUNCH(p, KT_FA_RED, (k_reduce_items<36>), grid_for(I.red_ch.n, 4), 128, 0, I.red_ch.n, I.red_ch.ch, I.red_ch.seg.p, I.red_ch.begin.p,
-                I.tgt_ptr.p, I.red_items.p, F.partP.p, F.red1P.p);
-    BA_LAUNCH(p, KT_FA_RED, (k_reduce_final<36>), grid_for(S.ndest, 4), 128, 0, S.ndest, I.red_ch.seg_first.p, F.red1P.p, p->Pacc.p);
-  }
-  BA_CUDA_TRY(cudaGetLastError());
+// Sums the partial blocks of one reduction list per target into out (n_targets blocks of NV doubles), in a fixed order.
+template <int NV>
+int reduce_partials(ba_cuda_problem* p, const ReduceList& R, int n_targets, double* out) {
+  if (R.ch.n > 0)
+    BA_LAUNCH(p, KT_FA_RED, (k_reduce_items<NV>), grid_for(R.ch.n, 4), 128, 0, R.ch.n, R.ch.ch, R.ch.seg.p, R.ch.begin.p, R.tgt_ptr.p,
+              R.items.p, R.part.p, R.red1.p);
+  BA_LAUNCH(p, KT_FA_RED, (k_reduce_final<NV>), grid_for(n_targets, 4), 128, 0, n_targets, R.ch.seg_first.p, R.red1.p, out);
   return BA_OK;
 }
 
-// r, J, cost, gradient norms at x AND the eliminated Schur system for the radius in scal[S_RADIUS]
-// (TrustRegionMinimizer::EvaluateGradientAndJacobian + SchurEliminator::Eliminate in one pass).
-// norms = true: iteration 0, computes the Jacobi scaling only.  grad_only = true: no further step can follow (the
-// iteration limit is reached), so only what the row of the progress table needs is computed: cost and gradient.
-// first = true: iteration 0 with Jacobi scaling in one pass (FA_FIRST): the point scaling is applied inside the pass, the
-// camera scaling to the reduced results.
-int sa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only, bool first);
-
-int fa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool norms, bool grad_only = false, bool first = false) {
-  const Structure& S = p->S;
-  FusedA& F = p->FA;
-  BA_TRY(fa_set_smem_attr(p));
-  if (p->use_strip) return sa_linearize(p, opt, grad_only, first);
-  fam_begin(p, F_JAC);
-  if (norms || first) {
-    BA_LAUNCH(p, KT_MISC, k_fill, grid_for(S.nf * 6, 256), 256, 0, p->sf.p, S.nf * 6, 1.0);
-    BA_LAUNCH(p, KT_MISC, k_fill, grid_for(S.ne * 3, 256), 256, 0, p->se.p, S.ne * 3, 1.0);
-  }
-  BA_TRY(build_tables(p, false));
+// Pass 1 on single tiles (ba_fused_a.cuh); n_cta: the number of CTAs, each leaving its cost / gradient partials in fa_part.
+int fa_pass1(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only, bool first, int& n_cta) {
+  const FusedA& F = p->FA;
   const FaParams P = fa_params(p, opt);
-  const int nt = F.n_tiles;
-  if (norms) {
-    BA_LAUNCH(p, KT_FA_P1L, (k_fa_pass1<FA_NORMS>), nt, F.threads, F.smem1(), P);
-    BA_TRY(fa_reduce(p, true, false));
-    BA_TRY(allreduce(p, F.camacc.p, (size_t)S.nf * FA_NVC, kNcclSum));
-    BA_LAUNCH(p, KT_MISC, (k_jacobi_scale<6, FA_NVC>), grid_for(S.nf * 6, 256), 256, 0, S.nf, F.camacc.p, p->sf.p);
-    BA_CUDA_TRY(cudaGetLastError());
-    fam_end(p, F_JAC);
-    return BA_OK;
-  }
-  BA_CUDA_TRY(cudaMemsetAsync(p->status.p, 0, sizeof(int), p->st));
-  if (grad_only) BA_LAUNCH(p, KT_FA_P1L, (k_fa_pass1<FA_GRAD>), nt, F.threads, F.smem1(), P);
-  else if (first) BA_LAUNCH(p, KT_FA_P1, (k_fa_pass1<FA_FIRST>), nt, F.threads, F.smem1(), P);
-  else BA_LAUNCH(p, KT_FA_P1, (k_fa_pass1<FA_FULL>), nt, F.threads, F.smem1(), P);
-  {
-    FoldJob J = {{P.cost_partial, P.g2_partial, P.gmax_partial, nullptr}, {S_COST, S_G2E, S_GMAXE, 0}, {0, 0, 1, 0}};
-    BA_LAUNCH(p, KT_FOLD, k_fold_multi, 3, 1024, 0, J, nt, p->scal.p);
-  }
-  fam_end(p, F_JAC);
-  fam_begin(p, F_SCHUR);
-  BA_TRY(fa_reduce(p, true, !grad_only));
-  fam_end(p, F_SCHUR);
-  const bool sx = sx_active(p);
-  if (p->world > 1) {  // camera sums and the shard-local gradient scalars in one collective; the partial blocks too when they travel sparse
-    fam_begin(p, F_COLL);
-    if (sx) BA_TRY(sx_exchange(p, F.camacc.p, !grad_only));
-    else BA_TRY(allreduce_with_grad_tail(p, F.camacc.p, (size_t)S.nf * FA_NVC));
-    fam_end(p, F_COLL);
-  }
-  if (first) {  // camera scaling from the (global) unscaled column norms, then everything reduced so far into scaled columns
-    BA_LAUNCH(p, KT_MISC, (k_jacobi_scale<6, FA_NVC>), grid_for(S.nf * 6, 256), 256, 0, S.nf, F.camacc.p, p->sf.p);
-    BA_LAUNCH(p, KT_MISC, k_fa_scale_cams, grid_for(S.nf * FA_NVC, 256), 256, 0, S.nf, p->sf.p, F.camacc.p);
-    if (sx) BA_LAUNCH(p, KT_MISC, k_sx_scale_blocks, grid_for((int64_t)p->R.nd * 36, 256), 256, 0, p->R.nd, p->R.fa.p, p->R.fb.p, p->sf.p, p->Sb.p);
-    else
-    BA_LAUNCH(p, KT_MISC, k_fa_scale_pairs, grid_for((int64_t)S.ndest * 36, 256), 256, 0, S.ndest, S.dest_fa.p, S.dest_fb.p, p->sf.p, p->Pacc.p);
-    BA_TRY(build_tables(p, false));   // pass 2 linearises with the scaled camera columns
-  }
-  const int gf = (int)grid_for(S.nf * 6, 256);
-  BA_LAUNCH(p, KT_GRADNORM, (k_gradient_norm<6, FA_NVC, 21>), gf, 256, 0, S.nf, p->f_act_ptr.p, p->xf.p, p->sf.p, F.camacc.p, p->bp0.p, p->bp1.p);
-  {
-    FoldJob J = {{p->bp0.p, p->bp1.p, nullptr, nullptr}, {S_GMAXF, S_G2F, 0, 0}, {1, 0, 0, 0}};
-    BA_LAUNCH(p, KT_FOLD, k_fold_multi, 2, 1024, 0, J, gf, p->scal.p);
-  }
-  BA_CUDA_TRY(cudaGetLastError());
+  n_cta = F.n_tiles;
+  if (grad_only) BA_LAUNCH(p, KT_FA_P1L, (k_fa_pass1<FA_GRAD>), n_cta, F.threads, F.smem1(), P);
+  else if (first) BA_LAUNCH(p, KT_FA_P1, (k_fa_pass1<FA_FIRST>), n_cta, F.threads, F.smem1(), P);
+  else BA_LAUNCH(p, KT_FA_P1, (k_fa_pass1<FA_FULL>), n_cta, F.threads, F.smem1(), P);
   return BA_OK;
 }
 
-// Strip path (ba_strip_a.cuh): one launch linearises, eliminates and accumulates the Schur products per strip; the
-// partial blocks (one per strip and camera pair / camera) are then summed in a fixed order.
-int sa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only, bool first) {
-  const Structure& S = p->S;
-  FusedA& F = p->FA;
-  StripA& A = p->SA;
-  fam_begin(p, F_JAC);
-  if (first) {
-    BA_LAUNCH(p, KT_MISC, k_fill, grid_for(S.nf * 6, 256), 256, 0, p->sf.p, S.nf * 6, 1.0);
-    BA_LAUNCH(p, KT_MISC, k_fill, grid_for(S.ne * 3, 256), 256, 0, p->se.p, S.ne * 3, 1.0);
-  }
-  BA_TRY(build_tables(p, false));
+// Pass 1 on strips (ba_strip_a.cuh): one CTA linearises, eliminates and accumulates the Schur products of a strip.
+int sa_pass1(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only, bool first, int& n_cta) {
+  const StripA& A = p->SA;
   const size_t ns = (size_t)A.n_strips;
   SaParams P;
   P.strips = A.strips.p; P.tiles = A.tiles.p; P.strip_cams = A.strip_cams.p; P.slot_out = A.slot_out.p;
@@ -727,8 +651,8 @@ int sa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only,
   P.segw = A.segw; P.cap_pos = A.cap_pos; P.pts_cap = A.pts_cap; P.tcs = A.tcs; P.ent_cap = A.ent_cap; P.pidx_cap = A.pidx_cap;
   P.xe = p->xe.p; P.se = p->se.p; P.tab_f = p->tab_f.p; P.radius = p->scal.p + S_RADIUS;
   P.min_diag = opt.min_lm_diagonal; P.max_diag = opt.max_lm_diagonal;
-  P.partP = A.partP.p; P.partC = A.partC.p; P.n_pout = A.n_pout;
-  P.Lz = F.Lz.p; P.se_out = p->se.p;
+  P.partP = A.red_pairs.part.p; P.partC = A.red_cams.part.p; P.n_pout = A.n_pout;
+  P.Lz = p->FA.Lz.p; P.se_out = p->se.p;
   P.cost_partial = p->fa_part.p; P.g2_partial = p->fa_part.p + ns; P.gmax_partial = p->fa_part.p + 2 * ns;
   P.status = p->status.p;
   P.dbg = env_int("BA_SA_DBG", 0, 7, 0);
@@ -740,10 +664,10 @@ int sa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only,
     BA_CUDA_TRY(cudaMemsetAsync(clk->p, 0, 8 * sizeof(unsigned long long), p->st));
     P.clocks = clk->p;
   }
-  BA_CUDA_TRY(cudaMemsetAsync(p->status.p, 0, sizeof(int), p->st));
-  if (first) BA_LAUNCH(p, KT_FA_P1, (k_sa_pass1<SA_FIRST>), A.n_strips, SA_NT, A.smem(), P);
-  else if (grad_only) BA_LAUNCH(p, KT_FA_P1L, (k_sa_pass1<SA_GRAD>), A.n_strips, SA_NT, A.smem(), P);
-  else BA_LAUNCH(p, KT_FA_P1, (k_sa_pass1<SA_FULL>), A.n_strips, SA_NT, A.smem(), P);
+  n_cta = A.n_strips;
+  if (first) BA_LAUNCH(p, KT_FA_P1, (k_sa_pass1<SA_FIRST>), n_cta, SA_NT, A.smem(), P);
+  else if (grad_only) BA_LAUNCH(p, KT_FA_P1L, (k_sa_pass1<SA_GRAD>), n_cta, SA_NT, A.smem(), P);
+  else BA_LAUNCH(p, KT_FA_P1, (k_sa_pass1<SA_FULL>), n_cta, SA_NT, A.smem(), P);
   if (P.clocks) {
     unsigned long long h[8];
     BA_CUDA_TRY(cudaMemcpyAsync(h, P.clocks, sizeof(h), cudaMemcpyDeviceToHost, p->st));
@@ -753,41 +677,77 @@ int sa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only,
                          "wait entries + barrier %.0f | B (own) %.0f | barrier after B %.0f | sum %.0f\n", h[0] / n, h[1] / n, h[2] / n, h[3] / n, h[4] / n,
                  h[5] / n, h[6] / n, (h[0] + h[1] + h[2] + h[3] + h[4] + h[5] + h[6]) / n);
   }
+  return BA_OK;
+}
+
+// Width of the per-camera record of the fused path: strips keep diag F^T F in a slot of its own (SA_NVC), single tiles
+// read it from the packed F^T F (FA_NVC).
+int fa_nvc(const ba_cuda_problem* p) { return p->use_strip ? SA_NVC : FA_NVC; }
+
+// r, J, cost, gradient norms at x AND the eliminated Schur system for the radius in scal[S_RADIUS]
+// (TrustRegionMinimizer::EvaluateGradientAndJacobian + SchurEliminator::Eliminate in one pass).
+// norms = true (single tiles only): iteration 0, computes the Jacobi scaling only.  grad_only = true: no further step can
+// follow (the iteration limit is reached), so only what the row of the progress table needs is computed: cost and
+// gradient.  first = true: iteration 0 with Jacobi scaling in one pass (FA_FIRST / SA_FIRST): the point scaling is applied
+// inside the pass, the camera scaling to the reduced results.  NVC: the camera record of the geometry (fa_nvc).
+template <int NVC>
+int fused_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool norms, bool grad_only, bool first) {
+  constexpr bool strip = NVC == SA_NVC;
+  constexpr int DIAG = strip ? 33 : -1;   // where diag F^T F sits in the record (-1: the packed diagonal)
+  const Structure& S = p->S;
+  FusedA& F = p->FA;
+  const ReduceList& red_cams = strip ? p->SA.red_cams : F.red_cams;
+  const ReduceList& red_pairs = strip ? p->SA.red_pairs : F.red_pairs;
+  BA_TRY(fa_set_smem_attr(p));
+  fam_begin(p, F_JAC);
+  if (norms || first) {
+    BA_LAUNCH(p, KT_MISC, k_fill, grid_for(S.nf * 6, 256), 256, 0, p->sf.p, S.nf * 6, 1.0);
+    BA_LAUNCH(p, KT_MISC, k_fill, grid_for(S.ne * 3, 256), 256, 0, p->se.p, S.ne * 3, 1.0);
+  }
+  BA_TRY(build_tables(p, false));
+  if (norms) {
+    BA_LAUNCH(p, KT_FA_P1L, (k_fa_pass1<FA_NORMS>), F.n_tiles, F.threads, F.smem1(), fa_params(p, opt));
+    BA_TRY(reduce_partials<NVC>(p, red_cams, (int)S.nf, F.camacc.p));
+    BA_CUDA_TRY(cudaGetLastError());
+    BA_TRY(allreduce(p, F.camacc.p, (size_t)S.nf * NVC, kNcclSum));
+    BA_LAUNCH(p, KT_MISC, (k_jacobi_scale<6, NVC, DIAG>), grid_for(S.nf * 6, 256), 256, 0, S.nf, F.camacc.p, p->sf.p);
+    BA_CUDA_TRY(cudaGetLastError());
+    fam_end(p, F_JAC);
+    return BA_OK;
+  }
+  BA_CUDA_TRY(cudaMemsetAsync(p->status.p, 0, sizeof(int), p->st));
+  int n_cta = 0;
+  BA_TRY(strip ? sa_pass1(p, opt, grad_only, first, n_cta) : fa_pass1(p, opt, grad_only, first, n_cta));
   {
-    FoldJob J = {{P.cost_partial, P.g2_partial, P.gmax_partial, nullptr}, {S_COST, S_G2E, S_GMAXE, 0}, {0, 0, 1, 0}};
-    BA_LAUNCH(p, KT_FOLD, k_fold_multi, 3, 1024, 0, J, A.n_strips, p->scal.p);
+    const double* part = p->fa_part.p;
+    FoldJob J = {{part, part + n_cta, part + 2 * (size_t)n_cta, nullptr}, {S_COST, S_G2E, S_GMAXE, 0}, {0, 0, 1, 0}};
+    BA_LAUNCH(p, KT_FOLD, k_fold_multi, 3, 1024, 0, J, n_cta, p->scal.p);
   }
   fam_end(p, F_JAC);
+  // the pair blocks are needed for a step, and on strips also for the scaling of iteration 0
+  const bool pairs = !grad_only || (strip && first);
   fam_begin(p, F_SCHUR);
-  if (A.red_ch_c.n > 0)
-    BA_LAUNCH(p, KT_FA_RED, (k_reduce_items<SA_NVC>), grid_for(A.red_ch_c.n, 4), 128, 0, A.red_ch_c.n, A.red_ch_c.ch, A.red_ch_c.seg.p,
-              A.red_ch_c.begin.p, A.tgt_ptr_c.p, A.red_items_c.p, A.partC.p, A.red1C.p);
-  BA_LAUNCH(p, KT_FA_RED, (k_reduce_final<SA_NVC>), grid_for(S.nf, 4), 128, 0, (int)S.nf, A.red_ch_c.seg_first.p, A.red1C.p, F.camacc.p);
-  if (!grad_only || first) {
-    if (A.red_ch_p.n > 0)
-      BA_LAUNCH(p, KT_FA_RED, (k_reduce_items<36>), grid_for(A.red_ch_p.n, 4), 128, 0, A.red_ch_p.n, A.red_ch_p.ch, A.red_ch_p.seg.p,
-                A.red_ch_p.begin.p, A.tgt_ptr_p.p, A.red_items_p.p, A.partP.p, A.red1P.p);
-    BA_LAUNCH(p, KT_FA_RED, (k_reduce_final<36>), grid_for(S.ndest, 4), 128, 0, S.ndest, A.red_ch_p.seg_first.p, A.red1P.p, p->Pacc.p);
-  }
+  BA_TRY(reduce_partials<NVC>(p, red_cams, (int)S.nf, F.camacc.p));
+  if (pairs) BA_TRY(reduce_partials<36>(p, red_pairs, S.ndest, p->Pacc.p));
   BA_CUDA_TRY(cudaGetLastError());
   fam_end(p, F_SCHUR);
   const bool sx = sx_active(p);
   if (p->world > 1) {  // camera sums and the shard-local gradient scalars in one collective; the partial blocks too when they travel sparse
     fam_begin(p, F_COLL);
-    if (sx) BA_TRY(sx_exchange(p, F.camacc.p, !grad_only || first));
-    else BA_TRY(allreduce_with_grad_tail(p, F.camacc.p, (size_t)S.nf * SA_NVC));
+    if (sx) BA_TRY(sx_exchange(p, F.camacc.p, pairs));
+    else BA_TRY(allreduce_with_grad_tail(p, F.camacc.p, (size_t)S.nf * NVC));
     fam_end(p, F_COLL);
   }
   if (first) {  // camera scaling from the (global) unscaled column norms, then everything reduced so far into scaled columns
-    BA_LAUNCH(p, KT_MISC, k_sa_jacobi_scale, grid_for(S.nf * 6, 256), 256, 0, S.nf, F.camacc.p, p->sf.p);
-    BA_LAUNCH(p, KT_MISC, k_sa_scale_cams, grid_for(S.nf * SA_NVC, 256), 256, 0, S.nf, p->sf.p, F.camacc.p);
+    BA_LAUNCH(p, KT_MISC, (k_jacobi_scale<6, NVC, DIAG>), grid_for(S.nf * 6, 256), 256, 0, S.nf, F.camacc.p, p->sf.p);
+    BA_LAUNCH(p, KT_MISC, (k_fa_scale_cams<NVC>), grid_for(S.nf * NVC, 256), 256, 0, S.nf, p->sf.p, F.camacc.p);
     if (sx) BA_LAUNCH(p, KT_MISC, k_sx_scale_blocks, grid_for((int64_t)p->R.nd * 36, 256), 256, 0, p->R.nd, p->R.fa.p, p->R.fb.p, p->sf.p, p->Sb.p);
     else
     BA_LAUNCH(p, KT_MISC, k_fa_scale_pairs, grid_for((int64_t)S.ndest * 36, 256), 256, 0, S.ndest, S.dest_fa.p, S.dest_fb.p, p->sf.p, p->Pacc.p);
     BA_TRY(build_tables(p, false));   // pass 2 linearises with the scaled camera columns
   }
   const int gf = (int)grid_for(S.nf * 6, 256);
-  BA_LAUNCH(p, KT_GRADNORM, (k_gradient_norm<6, SA_NVC, 21>), gf, 256, 0, S.nf, p->f_act_ptr.p, p->xf.p, p->sf.p, F.camacc.p, p->bp0.p, p->bp1.p);
+  BA_LAUNCH(p, KT_GRADNORM, (k_gradient_norm<6, NVC, 21>), gf, 256, 0, S.nf, p->f_act_ptr.p, p->xf.p, p->sf.p, F.camacc.p, p->bp0.p, p->bp1.p);
   {
     FoldJob J = {{p->bp0.p, p->bp1.p, nullptr, nullptr}, {S_GMAXF, S_G2F, 0, 0}, {1, 0, 0, 0}};
     BA_LAUNCH(p, KT_FOLD, k_fold_multi, 2, 1024, 0, J, gf, p->scal.p);
@@ -796,8 +756,16 @@ int sa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool grad_only,
   return BA_OK;
 }
 
+// Strips never take the separate scaling pass (norms): they always scale in one pass.
+int fa_linearize(ba_cuda_problem* p, const ba_cuda_options& opt, bool norms, bool grad_only = false, bool first = false) {
+  if (fa_nvc(p) == SA_NVC) return fused_linearize<SA_NVC>(p, opt, false, grad_only, first);
+  return fused_linearize<FA_NVC>(p, opt, norms, grad_only, first);
+}
+
 // RCS assembly + solve + (pass 2) back-substitution, model cost change, candidate and its cost
-int fa_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
+template <int NVC>
+int fused_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
+  constexpr int DIAG = NVC == SA_NVC ? 33 : -1;   // as in fused_linearize
   const Structure& S = p->S;
   FusedA& F = p->FA;
   const int64_t n = p->n_rcs();
@@ -823,24 +791,16 @@ int fa_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
   }
   fam_begin(p, F_SOLVE);
   if (pcg) {
-    if (p->use_strip)
-      BA_LAUNCH(p, KT_ASSEMBLE, k_sa_diag_rhs_bsr, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->R.diag.p, F.camacc.p, radius, opt.min_lm_diagonal,
-                opt.max_lm_diagonal, p->Sb.p, p->rhs.p);
-    else
-      BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_bsr, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->R.diag.p, F.camacc.p, FA_NVC, F.camacc.p + 27, FA_NVC,
-                radius, opt.min_lm_diagonal, opt.max_lm_diagonal, p->Sb.p, p->rhs.p);
+    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_bsr<DIAG>, grid_for(S.nf * 6, 128), 128, 0, S.nf, p->R.diag.p, F.camacc.p, NVC, F.camacc.p + 27, NVC,
+              radius, opt.min_lm_diagonal, opt.max_lm_diagonal, p->Sb.p, p->rhs.p);
     {
       LaunchScope scope(p, KT_RCS);
       BA_TRY(launch_pcg(p->pcg, p->R, p->Sb.p, p->rhs.p, p->yf.p, p->status.p, opt, p->st));
     }
     BA_CUDA_TRY(cudaMemcpyAsync(&p->h_pcg_iters, p->pcg.iters.p, sizeof(int), cudaMemcpyDeviceToHost, p->st));
   } else {
-    if (p->use_strip)
-      BA_LAUNCH(p, KT_ASSEMBLE, k_sa_diag_rhs_dense, grid_for(S.nf * 6, 128), 128, 0, S.nf, F.camacc.p, radius, opt.min_lm_diagonal,
-                opt.max_lm_diagonal, n, p->Sd.p, p->rhs.p);
-    else
-      BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_dense, grid_for(S.nf * 6, 128), 128, 0, S.nf, F.camacc.p, FA_NVC, F.camacc.p + 27, FA_NVC, radius,
-                opt.min_lm_diagonal, opt.max_lm_diagonal, n, p->Sd.p, p->rhs.p);
+    BA_LAUNCH(p, KT_ASSEMBLE, k_diag_rhs_dense<DIAG>, grid_for(S.nf * 6, 128), 128, 0, S.nf, F.camacc.p, NVC, F.camacc.p + 27, NVC, radius,
+              opt.min_lm_diagonal, opt.max_lm_diagonal, n, p->Sd.p, p->rhs.p);
     LaunchScope scope(p, KT_RCS);
     BA_TRY(dense_solve(p, n));
   }
@@ -863,6 +823,9 @@ int fa_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
   fam_end(p, F_UPDATE);
   return allreduce_step_scalars(p);
 }
+int fa_step(ba_cuda_problem* p, const ba_cuda_options& opt) {
+  return fa_nvc(p) == SA_NVC ? fused_step<SA_NVC>(p, opt) : fused_step<FA_NVC>(p, opt);
+}
 
 bool lm_fused(const ba_cuda_problem* p) { return p->model == 0 && p->use_fused && !p->lm.opt.force_generic_path; }
 
@@ -870,7 +833,7 @@ bool lm_fused(const ba_cuda_problem* p) { return p->model == 0 && p->use_fused &
 int sx_prepare(ba_cuda_problem* p) {
   const Structure& S = p->S;
   SparseExchange& X = p->SX;
-  X.on = false; X.world = p->world; X.nvc = p->use_strip ? SA_NVC : FA_NVC;
+  X.on = false; X.world = p->world; X.nvc = fa_nvc(p);
   if (!nccl().AllGather || !env_int("BA_SX", 0, 1, 1)) return BA_OK;
   cudaStream_t st = p->st;
   const int64_t nf = S.nf, nd = p->R.nd;

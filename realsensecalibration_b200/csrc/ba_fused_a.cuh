@@ -93,7 +93,16 @@ __global__ void k_fa_tile_desc(int n_tiles, const int64_t* __restrict__ tile_pt_
   out[t] = T;
 }
 
-// work items of one kind (pair items or camera items) and the static reduction lists over their partial blocks
+// The partial blocks of one kind (one per work item) and how they are summed per target, in a fixed order
+// (k_reduce_items, then k_reduce_final): the same lists for single tiles and for strips.
+struct ReduceList {
+  DVec<int32_t> items;          // item ids grouped by target (stable)
+  DVec<int64_t> tgt_ptr;        // n_targets + 1 into items
+  Chunks ch;                    // chunks over tgt_ptr
+  DVec<double> part, red1;      // partial blocks (per item), first-level sums (per chunk)
+};
+
+// work items of one kind (pair items or camera items)
 struct ItemSet {
   int64_t n_ent = 0;
   int n_items = 0, n_targets = 0, n_groups = 0;
@@ -102,9 +111,6 @@ struct ItemSet {
   DVec<int64_t> item_end;       // n_items
   DVec<int64_t> tile_item_ptr;  // n_tiles + 1
   DVec<int32_t> item_target;    // n_items: destination block / camera
-  DVec<int32_t> red_items;      // item ids grouped by target (stable)
-  DVec<int64_t> tgt_ptr;        // n_targets + 1 into red_items
-  Chunks red_ch;                // chunks over tgt_ptr
   // groups = distinct (tile, target)
   DVec<int64_t> group_ptr;      // n_groups + 1 into ent
   DVec<int32_t> group_target;   // n_groups
@@ -118,9 +124,10 @@ struct FusedA {
   DVec<int64_t> tile_pent_ptr;  // n_tiles + 1: the tile's slice of pairs.ent (entries are tile-major)
   DVec<int64_t> tile_cent_ptr;  // n_tiles + 1: the tile's slice of cams.ent
   ItemSet pairs, cams;
+  ReduceList red_pairs, red_cams; // over the items' partial blocks
   DVec<uint32_t> ob_meta;       // per observation: local point | camera slot << 16 (k_fa_ob_meta)
   DVec<FaTile> tiles;           // n_tiles descriptors
-  DVec<double> partP, partC, red1P, red1C, camacc, Lz;
+  DVec<double> camacc, Lz;
   // shared-memory geometry, from the maxima over the tiles of this problem (so that small tiles co-reside on an SM)
   int pts_cap = FA_TPTS;        // points of the fullest tile
   int tcam = FA_TCAM;           // camera tables staged per tile (cameras beyond are read from L2)
@@ -364,9 +371,9 @@ __global__ void k_fa_bank_order(int n_tiles, const int64_t* __restrict__ tile_it
 }
 
 // keys (tile * n_targets + target) with their entries -> sorted entries, groups, items of <= ch entries ordered by
-// (tile, descending length), reduction lists
+// (tile, descending length), the reduction lists R over the items
 template <typename K>
-inline int build_items(ItemSet& I, DVec<K>& keys, DVec<int32_t>& vals, int64_t n, int n_tiles, int64_t n_targets, int ch,
+inline int build_items(ItemSet& I, ReduceList& R, DVec<K>& keys, DVec<int32_t>& vals, int64_t n, int n_tiles, int64_t n_targets, int ch,
                        bool is_pair, const GroupDecode& D, cudaStream_t st) {
   I.n_ent = n; I.n_targets = (int)n_targets;
   FaLap L(st);
@@ -423,8 +430,8 @@ inline int build_items(ItemSet& I, DVec<K>& keys, DVec<int32_t>& vals, int64_t n
   if (env_int("BA_FA_BANK_ORDER", 0, 1, 1))
     k_fa_bank_order<<<grid_for(n_tiles, 4), 128, 0, st>>>(n_tiles, I.tile_item_ptr.p, I.item_begin.p, I.item_end.p, I.ent.p, is_pair ? 1 : 0);
   L.lap("items: bank order");
-  BA_TRY(sort_to_csr(I.item_target.p, iota.p, ni, n_targets, I.tgt_ptr, I.red_items, st));
-  BA_TRY(build_chunks(I.red_ch, I.tgt_ptr.p, (int)n_targets, FA_CH_RED, st));
+  BA_TRY(sort_to_csr(I.item_target.p, iota.p, ni, n_targets, R.tgt_ptr, R.items, st));
+  BA_TRY(build_chunks(R.ch, R.tgt_ptr.p, (int)n_targets, FA_CH_RED, st));
   L.lap("items: reduction lists");
   BA_CUDA_TRY(cudaStreamSynchronize(st));
   BA_CUDA_TRY(cudaGetLastError());
@@ -487,7 +494,7 @@ inline int build_fused_a_tobs(FusedA& F, const Structure& S, cudaStream_t st, in
     k_fa_cam_fill<<<grid_for(nb, 256), 256, 0, st>>>(S.ob_e.p, S.ob_f0.p, nb, nf, S.e_ptr.p, tile_of_pt.p, F.tile_pt_ptr.p, keys.p, vals.p);
     GroupDecode D;
     D.n_targets = (uint64_t)nf; D.key_bits = bits_for((uint64_t)F.n_tiles * (uint64_t)nf);
-    BA_TRY(build_items<uint64_t>(F.cams, keys, vals, nb, F.n_tiles, nf, F.ch_cam, false, D, st));
+    BA_TRY(build_items<uint64_t>(F.cams, F.red_cams, keys, vals, nb, F.n_tiles, nf, F.ch_cam, false, D, st));
     const int ng = F.cams.n_groups;
     BA_TRY(group_tile.alloc(ng)); BA_TRY(F.ob_meta.alloc(nb));
     // group -> tile from the tile_group_ptr CSR (groups are tile-major)
@@ -524,7 +531,7 @@ inline int build_fused_a_tobs(FusedA& F, const Structure& S, cudaStream_t st, in
       D.mode = 1; D.sb = sb; D.key_bits = 2 * sb + tb;
       D.tile_cam_ptr = F.cams.tile_group_ptr.p; D.tile_cams = F.cams.group_target.p;
       D.dh_keys = S.dh_keys.p; D.dh_val = S.dh_val.p; D.dh_mask = S.dh_mask; D.dh_shift = S.dh_shift;
-      BA_TRY(build_items<uint32_t>(F.pairs, keys, vals, np, F.n_tiles, S.ndest, F.ch_pair, true, D, st));
+      BA_TRY(build_items<uint32_t>(F.pairs, F.red_pairs, keys, vals, np, F.n_tiles, S.ndest, F.ch_pair, true, D, st));
     } else {
       DVec<uint64_t> keys;
       BA_TRY(keys.alloc(np));
@@ -533,7 +540,7 @@ inline int build_fused_a_tobs(FusedA& F, const Structure& S, cudaStream_t st, in
                                                         vals.p);
       L.lap("pair fill");
       D.key_bits = bits_for((uint64_t)F.n_tiles * (uint64_t)S.ndest);
-      BA_TRY(build_items<uint64_t>(F.pairs, keys, vals, np, F.n_tiles, S.ndest, F.ch_pair, true, D, st));
+      BA_TRY(build_items<uint64_t>(F.pairs, F.red_pairs, keys, vals, np, F.n_tiles, S.ndest, F.ch_pair, true, D, st));
     }
   }
   {  // per-tile slices of the entry lists; shared-memory geometry from the fullest tile
@@ -562,8 +569,8 @@ inline int build_fused_a_tobs(FusedA& F, const Structure& S, cudaStream_t st, in
   BA_TRY(F.tiles.alloc((size_t)F.n_tiles));
   k_fa_tile_desc<<<grid_for(F.n_tiles, 256), 256, 0, st>>>(F.n_tiles, F.tile_pt_ptr.p, S.e_ptr.p, F.cams.tile_group_ptr.p, F.tile_pent_ptr.p,
                                                           F.tile_cent_ptr.p, F.pairs.tile_item_ptr.p, F.cams.tile_item_ptr.p, F.tiles.p);
-  BA_TRY(F.partP.alloc((size_t)F.pairs.n_items * 36)); BA_TRY(F.partC.alloc((size_t)F.cams.n_items * FA_NVC));
-  BA_TRY(F.red1P.alloc((size_t)F.pairs.red_ch.n * 36)); BA_TRY(F.red1C.alloc((size_t)F.cams.red_ch.n * FA_NVC));
+  BA_TRY(F.red_pairs.part.alloc((size_t)F.pairs.n_items * 36)); BA_TRY(F.red_cams.part.alloc((size_t)F.cams.n_items * FA_NVC));
+  BA_TRY(F.red_pairs.red1.alloc((size_t)F.red_pairs.ch.n * 36)); BA_TRY(F.red_cams.red1.alloc((size_t)F.red_cams.ch.n * FA_NVC));
   BA_TRY(F.camacc.alloc((size_t)nf * FA_NVC + 2 + 64));  // tail: shard-local gradient scalars (ba_cuda.cu, kMaxWorld)
   BA_TRY(F.Lz.alloc((size_t)ne * 9));
   BA_CUDA_TRY(cudaStreamSynchronize(st));
@@ -1206,19 +1213,23 @@ __global__ void __launch_bounds__(FA_JAC_THREADS, 4) k_fa_jac(FaParams P) {
   if (tid == 0) P.cost_partial[tile] = sq;
 }
 
-// FA_FIRST: the reduced camera-side results of the unscaled pass, brought to Jacobi-scaled camera columns
+// FA_FIRST / SA_FIRST: the reduced camera-side results of the unscaled pass, brought to Jacobi-scaled camera columns
+// (NVC = FA_NVC on tiles; SA_NVC on strips, whose tail holds diag F^T F)
+template <int NVC>
 __global__ void k_fa_scale_cams(int64_t nf, const double* __restrict__ sf, double* __restrict__ camacc) {
   const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (t >= nf * FA_NVC) return;
-  const int64_t c = t / FA_NVC;
-  const int v = (int)(t % FA_NVC);
+  if (t >= nf * NVC) return;
+  const int64_t c = t / NVC;
+  const int v = (int)(t % NVC);
   double f;
   if (v < 21) {  // packed upper (a <= b) of F^T F
     int a = 0, rem = v;
     while (rem >= 6 - a) { rem -= 6 - a; ++a; }
     f = sf[6 * c + a] * sf[6 * c + a + rem];
-  } else {
+  } else if (NVC == 33 || v < 33) {
     f = sf[6 * c + (v - 21) % 6];   // F^T r, sum of v
+  } else {
+    f = sf[6 * c + (v - 33)] * sf[6 * c + (v - 33)];   // diag F^T F (strips)
   }
   camacc[t] *= f;
 }

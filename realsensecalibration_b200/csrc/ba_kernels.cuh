@@ -807,7 +807,9 @@ __global__ void k_assemble_dense(int ndest, const int32_t* __restrict__ dest_fa,
   if (t < (int64_t)ndest * 36) d_assemble_dense(t, dest_fa, dest_fb, P, Q, n, S);
 }
 
-// After the (optional) cross-GPU sum: add F^T F diagonal blocks and the LM diagonal D_f^2, form the rhs.
+// After the (optional) cross-GPU sum: add F^T F diagonal blocks and the LM diagonal D_f^2, form the rhs.  DOFF as in
+// k_diag_rhs_bsr (ba_rcs.cuh).
+template <int DOFF = -1>
 __device__ __forceinline__ void d_diag_rhs_dense(int64_t t, const double* __restrict__ HG, int hg_stride, const double* __restrict__ vsum,
                                                  int v_stride, const double* __restrict__ radius_p, double min_diag, double max_diag,
                                                  int64_t n /* row stride */, double* __restrict__ S, double* __restrict__ rhs) {
@@ -817,16 +819,17 @@ __device__ __forceinline__ void d_diag_rhs_dense(int64_t t, const double* __rest
 #pragma unroll
   for (int b = 0; b < 6; ++b) {
     double h = H[a <= b ? sym_idx6(a, b) : sym_idx6(b, a)];
-    if (a == b) { const double d = sqrt(fmin(fmax(h, min_diag), max_diag) / *radius_p); h += d * d; }
+    if (a == b) { const double d = sqrt(fmin(fmax(DOFF < 0 ? h : H[DOFF + a], min_diag), max_diag) / *radius_p); h += d * d; }
     S[(6 * f + a) * n + 6 * f + b] += h;
   }
   rhs[t] = H[21 + a] - vsum[f * v_stride + a];
 }
+template <int DOFF = -1>
 __global__ void k_diag_rhs_dense(int64_t nf, const double* __restrict__ HG, int hg_stride, const double* __restrict__ vsum,
                                  int v_stride, const double* __restrict__ radius_p, double min_diag, double max_diag, int64_t n,
                                  double* __restrict__ S, double* __restrict__ rhs) {
   const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (t < nf * 6) d_diag_rhs_dense(t, HG, hg_stride, vsum, v_stride, radius_p, min_diag, max_diag, n, S, rhs);
+  if (t < nf * 6) d_diag_rhs_dense<DOFF>(t, HG, hg_stride, vsum, v_stride, radius_p, min_diag, max_diag, n, S, rhs);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -976,18 +979,19 @@ k_gradient_norm(int64_t nblk, const int64_t* __restrict__ ptr, const double* __r
   if (threadIdx.x == 0) { p_max[blockIdx.x] = mx; p_sq[blockIdx.x] = sq; }
 }
 
-// Jacobi scaling s = 1 / (1 + sqrt(|column|^2)) from the packed normal-equation diagonals (iteration 0 only).
-template <int W, int NVB>
+// Jacobi scaling s = 1 / (1 + sqrt(|column|^2)) from the packed normal-equation diagonals (iteration 0 only), or, DOFF >= 0,
+// from the W column norms stored at src[DOFF..] of each block.
+template <int W, int NVB, int DOFF = -1>
 __device__ __forceinline__ void d_jacobi_scale(int64_t t, const double* __restrict__ src, double* __restrict__ s) {
   const int64_t b = t / W;
   const int k = (int)(t % W);
-  const int di = k * W - k * (k - 1) / 2;  // packed index of (k,k)
+  const int di = DOFF < 0 ? k * W - k * (k - 1) / 2 : DOFF + k;  // packed index of (k,k), or a separate diagonal
   s[t] = 1.0 / (1.0 + sqrt(src[b * NVB + di]));
 }
-template <int W, int NVB>
+template <int W, int NVB, int DOFF = -1>
 __global__ void k_jacobi_scale(int64_t nblk, const double* __restrict__ src, double* __restrict__ s) {
   const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (t < nblk * W) d_jacobi_scale<W, NVB>(t, src, s);
+  if (t < nblk * W) d_jacobi_scale<W, NVB, DOFF>(t, src, s);
 }
 
 __global__ void k_fill(double* a, int64_t n, double v) {

@@ -80,6 +80,9 @@ __global__ void k_assemble_bsr(int ndest, const int32_t* __restrict__ l2g, const
   Sb[(int64_t)l2g[d] * 36 + q] = (Q ? Q[t] : 0.0) - P[t];
 }
 
+// diagonal block += F^T F + D_f^2, rhs = F^T r - sum v.  DOFF >= 0: the LM diagonal is taken from diag F^T F at HG[DOFF..]
+// (the strip record, whose packed block is F^T (I - U^T U) F); -1: from the packed block itself.
+template <int DOFF = -1>
 __global__ void k_diag_rhs_bsr(int64_t nf, const int32_t* __restrict__ diag, const double* __restrict__ HG, int hg_stride,
                                const double* __restrict__ vsum, int v_stride, const double* __restrict__ radius_p, double min_diag, double max_diag, double* __restrict__ Sb,
                                double* __restrict__ rhs) {
@@ -92,7 +95,7 @@ __global__ void k_diag_rhs_bsr(int64_t nf, const int32_t* __restrict__ diag, con
 #pragma unroll
   for (int b = 0; b < 6; ++b) {
     double h = H[a <= b ? sym_idx6(a, b) : sym_idx6(b, a)];
-    if (a == b) { const double d = sqrt(fmin(fmax(h, min_diag), max_diag) / *radius_p); h += d * d; }
+    if (a == b) { const double d = sqrt(fmin(fmax(DOFF < 0 ? h : H[DOFF + a], min_diag), max_diag) / *radius_p); h += d * d; }
     B[a * 6 + b] += h;
   }
   rhs[t] = H[21 + a] - vsum[f * v_stride + a];

@@ -71,11 +71,7 @@ struct StripA {
   DVec<int32_t> ent;            // per tile: entries by owner slot
   DVec<uint16_t> seg;           // [n_tiles][segw]: first entry of every owner slot
   DVec<uint32_t> ob_meta;       // per sorted observation: local point | camera slot << 16 (pass 2, k_fa_jac)
-  // reduction lists over the partial blocks (k_reduce_items / k_reduce_final)
-  DVec<int32_t> red_items_p, red_items_c;
-  DVec<int64_t> tgt_ptr_p, tgt_ptr_c;
-  Chunks red_ch_p, red_ch_c;
-  DVec<double> partP, partC, red1P, red1C;
+  ReduceList red_pairs, red_cams; // the partial blocks per strip and camera pair / camera
   size_t smem() const {
     size_t b = ((size_t)cap_pos * SA_REC + (size_t)tcs * TAB + 2 * (size_t)sa_xs_len(pts_cap)) * 8;
     b += (size_t)cap_pos * 16 + (size_t)cap_pos * 4 + (size_t)pidx_cap * 2 + (size_t)ent_cap * 4 + (size_t)segw * 2 + 64;
@@ -883,15 +879,15 @@ inline int build_strip_a_geom(StripA& A, FusedA& F, const Structure& S, const do
     const int64_t nmax = std::max(n_pblocks, A.n_cout);
     BA_TRY(iota.alloc((size_t)nmax));
     k_iota<<<grid_for(nmax, 256), 256, 0, st>>>(iota.p, nmax, 0);
-    BA_TRY(sort_to_csr(ptarget.p, iota.p, n_pblocks, S.ndest, A.tgt_ptr_p, A.red_items_p, st));
-    BA_TRY(build_chunks(A.red_ch_p, A.tgt_ptr_p.p, S.ndest, FA_CH_RED, st));
-    BA_TRY(sort_to_csr(ctarget.p, iota.p, A.n_cout, nf, A.tgt_ptr_c, A.red_items_c, st));
-    BA_TRY(build_chunks(A.red_ch_c, A.tgt_ptr_c.p, (int)nf, FA_CH_RED, st));
+    BA_TRY(sort_to_csr(ptarget.p, iota.p, n_pblocks, S.ndest, A.red_pairs.tgt_ptr, A.red_pairs.items, st));
+    BA_TRY(build_chunks(A.red_pairs.ch, A.red_pairs.tgt_ptr.p, S.ndest, FA_CH_RED, st));
+    BA_TRY(sort_to_csr(ctarget.p, iota.p, A.n_cout, nf, A.red_cams.tgt_ptr, A.red_cams.items, st));
+    BA_TRY(build_chunks(A.red_cams.ch, A.red_cams.tgt_ptr.p, (int)nf, FA_CH_RED, st));
     BA_CUDA_TRY(cudaStreamSynchronize(st));
   }
   Lp.lap("strip: reduction lists");
-  BA_TRY(A.partP.alloc((size_t)n_pblocks * 36)); BA_TRY(A.partC.alloc((size_t)A.n_cout * SA_NVC));
-  BA_TRY(A.red1P.alloc((size_t)A.red_ch_p.n * 36)); BA_TRY(A.red1C.alloc((size_t)A.red_ch_c.n * SA_NVC));
+  BA_TRY(A.red_pairs.part.alloc((size_t)n_pblocks * 36)); BA_TRY(A.red_cams.part.alloc((size_t)A.n_cout * SA_NVC));
+  BA_TRY(A.red_pairs.red1.alloc((size_t)A.red_pairs.ch.n * 36)); BA_TRY(A.red_cams.red1.alloc((size_t)A.red_cams.ch.n * SA_NVC));
   // 8. the tile structure pass 2 and k_fa_jac run on
   F.n_tiles = nt; F.tobs = tobs; F.kmax = A.kmax; F.cap = std::max(A.nobs_cap, 1);
   F.threads = SA_NT; F.threads2 = env_int("BA_FA_THREADS2", 32, FA_MAX_THREADS, tobs >= 640 ? 256 : 128) / 32 * 32;
@@ -1296,63 +1292,6 @@ __global__ void __launch_bounds__(SA_NT, 1) k_sa_pass1(SaParams P) {
     fa_block_reduce(v, mx, 3, red);
     if (tid == 0) { P.cost_partial[blockIdx.x] = v[0]; P.g2_partial[blockIdx.x] = v[1]; P.gmax_partial[blockIdx.x] = v[2]; }
   }
-}
-
-// FA_FIRST: the reduced camera-side results of the unscaled pass, brought to Jacobi-scaled camera columns (SA_NVC layout)
-__global__ void k_sa_scale_cams(int64_t nf, const double* __restrict__ sf, double* __restrict__ camacc) {
-  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (t >= nf * SA_NVC) return;
-  const int64_t c = t / SA_NVC;
-  const int v = (int)(t % SA_NVC);
-  double f;
-  if (v < 21) {  // packed upper (a <= b)
-    int a = 0, rem = v;
-    while (rem >= 6 - a) { rem -= 6 - a; ++a; }
-    f = sf[6 * c + a] * sf[6 * c + a + rem];
-  } else if (v < 33) {
-    f = sf[6 * c + (v - 21) % 6];   // F^T r, sum of v
-  } else {
-    f = sf[6 * c + (v - 33)] * sf[6 * c + (v - 33)];   // diag F^T F
-  }
-  camacc[t] *= f;
-}
-// Jacobi scaling of the cameras from the unscaled column norms (the diag F^T F part of the SA_NVC record)
-__global__ void k_sa_jacobi_scale(int64_t nf, const double* __restrict__ camacc, double* __restrict__ sf) {
-  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (t >= nf * 6) return;
-  sf[t] = 1.0 / (1.0 + sqrt(camacc[(t / 6) * SA_NVC + 33 + (t % 6)]));
-}
-// diagonal block (already holding -P_ff = 0 here) += F^T (I - U^T U) F + D_f^2, rhs = F^T r - sum v
-__global__ void k_sa_diag_rhs_bsr(int64_t nf, const int32_t* __restrict__ diag, const double* __restrict__ camacc, const double* __restrict__ radius_p,
-                                  double min_diag, double max_diag, double* __restrict__ Sb, double* __restrict__ rhs) {
-  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (t >= nf * 6) return;
-  const int64_t f = t / 6;
-  const int a = (int)(t % 6);
-  const double* H = camacc + f * SA_NVC;
-  double* B = Sb + (int64_t)diag[f] * 36;
-#pragma unroll
-  for (int b = 0; b < 6; ++b) {
-    double h = H[a <= b ? sym_idx6(a, b) : sym_idx6(b, a)];
-    if (a == b) { const double d = sqrt(fmin(fmax(H[33 + a], min_diag), max_diag) / *radius_p); h += d * d; }
-    B[a * 6 + b] += h;
-  }
-  rhs[t] = H[21 + a] - H[27 + a];
-}
-__global__ void k_sa_diag_rhs_dense(int64_t nf, const double* __restrict__ camacc, const double* __restrict__ radius_p, double min_diag,
-                                    double max_diag, int64_t n, double* __restrict__ Sd, double* __restrict__ rhs) {
-  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (t >= nf * 6) return;
-  const int64_t f = t / 6;
-  const int a = (int)(t % 6);
-  const double* H = camacc + f * SA_NVC;
-#pragma unroll
-  for (int b = 0; b < 6; ++b) {
-    double h = H[a <= b ? sym_idx6(a, b) : sym_idx6(b, a)];
-    if (a == b) { const double d = sqrt(fmin(fmax(H[33 + a], min_diag), max_diag) / *radius_p); h += d * d; }
-    Sd[(6 * f + a) * n + 6 * f + b] += h;
-  }
-  rhs[t] = H[21 + a] - H[27 + a];
 }
 
 }  // namespace ba
